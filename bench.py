@@ -17,6 +17,10 @@ all-gather per pcut and one all-reduce of the packed tallies per ion (NCCL insid
   roofline     the transport kernel against the FP64 pipe: steps x 185 flop (SURVEY 8d / DESIGN.md) / kernel time,
                over a DFMA peak measured live on this GPU (MEASURED_PEAKS.json has no FP64 entry).
   cpu_baseline the CPU oracle (C restatement; Julia is not available) on a bounded sample, all host threads.
+
+--dump-outputs DIR writes what the last timed step handed back to its caller (per ion: the pcut counts of mcs_run_ion, the
+tallies, scalars and counters of mcs_end_ion) as DIR/ion<i>_<name>.npy in float64, so that two builds run with the same
+arguments, which see the same inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -38,6 +42,10 @@ FLOP_PER_STEP = 185.0  # SURVEY.md 8d, Appendix D; restated in DESIGN.md
 # .ncu-rep; tools/profile.sh).  Reported only when the capture matches the workload and the particle count; else null.
 TRAFFIC_FILE = os.path.join(ROOT, "profiles", "r02_traffic.json")
 METRIC = "scattering_steps_per_sec"
+DUMP_BYTES = 64_000_000
+DUMP_TALLIES = ("pxx_flux", "pxz_flux", "energy_flux", "psd", "num_crossings", "esc_psd_feb_upstream", "esc_psd_feb_downstream",
+                "esc_energy_eff", "esc_num_eff", "weight_coupled", "spectra_coupled", "energy_transfer_pool", "spectra_sf",
+                "spectra_pf")
 
 
 def measured_traffic(workload, n_per_pcut):
@@ -79,6 +87,37 @@ def workload_config(workload, run, n_per_pcut, extra=None):
     if extra:
         c.update(extra)
     return c
+
+
+def step_outputs(res):
+    """name -> array: per ion of one step, what its caller receives from mcs_run_ion and mcs_end_ion."""
+    out = {}
+    for i, r in res.items():
+        t = r["t"]
+        arrays = {"n_used": r["n_used"], "n_saved": r["n_saved"], **{nm: getattr(t, nm) for nm in DUMP_TALLIES},
+                  **t.scalars, **t.stats}
+        out.update({f"ion{i}_{k}": v for k, v in arrays.items()})
+    return out
+
+
+def dump_outputs(path, arrays, limit=DUMP_BYTES):
+    """Writes each array as <path>/<name>.npy in float64.  When together they would exceed `limit` bytes, every array of more
+    than 1 MB keeps the same fraction of its entries, at flat indices drawn with a fixed seed: two runs of the same shapes
+    keep the same entries."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    limit -= 1024 * len(arrays)  # .npy headers
+    big = sorted(k for k, v in arrays.items() if v.nbytes > 1 << 20)
+    small = sum(v.nbytes for k, v in arrays.items() if k not in big)
+    total = small + sum(arrays[k].nbytes for k in big)
+    if total > limit:
+        frac = (limit - small) / (total - small)
+        for k in big:
+            v = arrays[k].ravel()
+            idx = np.random.default_rng(0).choice(v.size, int(v.size * frac), replace=False)
+            arrays[k] = v[np.sort(idx)]
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 class ClockSampler:
@@ -226,7 +265,13 @@ def main():
     ap.add_argument("--no-verify", action="store_true", help="skip the N-rank vs 1-rank check that precedes a multi-GPU run")
     ap.add_argument("--generate-in-library", action="store_true",
                     help="SURVEY 8(f2): hand init_pop to the library in run-length form instead of copying host arrays")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one to DIR/<name>.npy (float64, <= 64 MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm (--impl b200)")
     # stdout carries exactly one JSON line: libraries that write to fd 1 (NCCL prints its version there) go to stderr
     sys.stdout.flush()
     out_fd = os.dup(1)
@@ -342,7 +387,8 @@ def main():
             t = eng.end_ion(want_psd=True, want_log=False)
             pool = pool + t.energy_transfer_pool
             t1 = eng.timing()
-            res[i_ion] = dict(t=t, n_run=n_run, steps=t.stats["n_helix_steps"] + t.stats["n_retro_steps"],
+            res[i_ion] = dict(t=t, n_run=n_run, n_used=n_used, n_saved=n_saved,
+                              steps=t.stats["n_helix_steps"] + t.stats["n_retro_steps"],
                               loop_ms=t1["ion_loop_ms"] - t0["ion_loop_ms"], kern_ms=t1["transport_ms"] - t0["transport_ms"],
                               d2h=sum(getattr(t, nm).nbytes for nm in D2H_FIELDS) + 8 * 8 + 24 * 8)
         return res
@@ -357,19 +403,23 @@ def main():
     wall, res = 0.0, {}
     sp_steps = {i: 0.0 for i in ions}
     sp_ms = {i: 0.0 for i in ions}
-    barrier()
-    for _ in range(a.steps):
-        flush.fill_(1)  # L2 flush between timed iterations (not timed)
+    try:  # a failing step must not leave the nvidia-smi sampler running
         barrier()
-        t0 = time.perf_counter()
-        res = one_step()
-        torch.cuda.synchronize()
-        wall += time.perf_counter() - t0
-        for i in ions:
-            sp_steps[i] += res[i]["steps"]   # already summed over ranks by the all-reduce of mcs_end_ion
-            sp_ms[i] += res[i]["loop_ms"]
-    barrier()
-    clocks = sampler.stop() if sampler else None
+        for _ in range(a.steps):
+            flush.fill_(1)  # L2 flush between timed iterations (not timed)
+            barrier()
+            t0 = time.perf_counter()
+            res = one_step()
+            torch.cuda.synchronize()
+            wall += time.perf_counter() - t0
+            for i in ions:
+                sp_steps[i] += res[i]["steps"]   # already summed over ranks by the all-reduce of mcs_end_ion
+                sp_ms[i] += res[i]["loop_ms"]
+        barrier()
+    finally:
+        clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, step_outputs(res))
     tm = eng.timing()
     steps_total = float(sum(sp_steps.values()))      # global, all timed steps
     steps_per_iter = steps_total / a.steps

@@ -52,15 +52,18 @@ def test_default_config_identical(olib):
 
 
 def test_no_cpu_fallback_without_gpu():
-    """On a box without a GPU the product must fail loudly, never compute on the CPU."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    lib = mcs_b200.load_cuda_library()
-    cfg = abi.default_config(lib)
-    cfg.n_grid, cfg.num_psd_mom_bins, cfg.num_psd_theta_bins = 99, 171, 159
-    with pytest.raises(abi.McsError, match="no CUDA device"):
-        abi.Engine(lib, cfg)
+    """Where no GPU is visible the product must fail loudly, never compute on the CPU.  Checked in a child process that sees
+    no device (CUDA_VISIBLE_DEVICES empty), so that it also holds on a machine with GPUs."""
+    import subprocess
+    import sys
+    code = ("import mcs_b200\nfrom mcs_b200 import abi\n"
+            "lib = mcs_b200.load_cuda_library()\ncfg = abi.default_config(lib)\n"
+            "cfg.n_grid, cfg.num_psd_mom_bins, cfg.num_psd_theta_bins = 99, 171, 159\n"
+            "try:\n    abi.Engine(lib, cfg)\nexcept abi.McsError as e:\n    print(e)\n")
+    out = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 0, out.stderr
+    assert "no CUDA device" in out.stdout, out.stdout
 
 
 def test_package_does_not_import_oracle():
