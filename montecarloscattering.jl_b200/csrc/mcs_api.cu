@@ -321,11 +321,8 @@ extern "C" int mcs_create(const McsConfig* cfg, McsHandle** out) {
     t.tg = h->d_tg; t.tpx = h->d_tpx; t.tpt = h->d_tpt; t.tw = h->d_tw; t.na_cr = cfg->na_cr;
     t.block_partials = h->d_partials;
     {
-        double2 az[AZ_N];  // host libm: sine and cosine of the bin centres of the scattering azimuth
-        for (int k = 0; k < AZ_N; k++) {
-            const double a = -PI + TWO_PI * (k + 0.5) / AZ_N;
-            az[k].x = sin(a); az[k].y = cos(a);
-        }
+        double2 az[AZ_N];  // sine and cosine of the bin centres of the scattering azimuth
+        az_table(az);
         cudaError_t e2 = cudaMemcpyAsync(h->d_az, az, sizeof az, cudaMemcpyHostToDevice, h->stream);
         if (e2 == cudaSuccess) e2 = cudaStreamSynchronize(h->stream);
         if (e2 != cudaSuccess) { mcs_destroy(h); return fail(MCS_ERR_CUDA, "CUDA error: %s", cudaGetErrorString(e2)); }

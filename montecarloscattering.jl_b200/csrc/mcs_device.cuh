@@ -228,8 +228,9 @@ __device__ __forceinline__ void count(const DevParams& P, int which, unsigned lo
 // the multiples of 2^(ACC_ELO + 32 k): a contribution m * 2^e (m its 53-bit significand) is cut at the word boundaries into
 // at most three pieces of < 2^32 and each piece is ADDED to its word with an integer atomic.  Integer adds commute and the
 // words have 31 bits of headroom (2^31 contributions per cell before a carry could be lost), so the words — and the double
-// they are folded into at the end of the ion — do not depend on the order of the adds: bitwise identical run to run, for
-// any schedule and any number of GPUs (the per-rank words are summed with an integer all-reduce).  The window is fixed:
+// they are folded into at the end of the ion, the correctly rounded value of the integer they hold — do not depend on the
+// order of the adds: bitwise identical run to run, for any schedule and any number of GPUs (the per-rank words are summed
+// with an integer all-reduce).  The window is fixed:
 // values in [2^-157, 2^98) keep all 53 bits, smaller ones lose their low bits below 2^-210, anything else is counted as an
 // error.  (Weights here are ~1e-6 at injection and shrink by up to ~1e-20 in a deep pcut ladder; 1/v >= 3e-11.)
 constexpr int ACC_D = 10;
@@ -1407,7 +1408,9 @@ constexpr double COS_AT_LIMIT = 1.4901161193847656e-08;  // sqrt(1 - prevfloat(1
 // sin and cos of the scattering azimuth phi_s = 2 pi u - pi (scattering.jl:71) for u = w / 2^53, w the 53-bit random
 // integer (hi:lo >> 11): the top 8 bits of w pick a table entry {sin A_k, cos A_k}, A_k = -pi + 2 pi (k + 1/2) / 256, the
 // other 45 bits the offset |t| <= pi/256 from it, whose sine and cosine need three terms each; angle addition.  12 FP64
-// operations and 6 constants instead of 26 and 16 for a general sincos; error <= 1.5 ulp of 1.
+// operations and 6 constants instead of 26 and 16 for a general sincos; error <= 2.5 ulp of 1 against the exact azimuth
+// (measured 2.45 on B200, tests/test_device_units.py), up to 2.36 of which is the table's: az_table rounds the bin centre to
+// double before libm sees it.
 __device__ __forceinline__ void az_sincos(const double2* __restrict__ tab, uint32_t hi, uint32_t lo, double& s_out, double& c_out) {
     const uint32_t k = hi >> 24;
     // f = bits 44..0 of w: bits 23..11 of hi (13 bits) above bits 31..11 of lo... as an exact double via the 2^52 trick
@@ -1424,6 +1427,13 @@ __device__ __forceinline__ void az_sincos(const double2* __restrict__ tab, uint3
     const double2 e = tab[k];
     s_out = fma(e.x, ct, e.y * st);
     c_out = fma(e.y, ct, -(e.x * st));
+}
+// the table az_sincos reads (DevParams.az_tab), built on the host with its libm
+__host__ inline void az_table(double2 tab[AZ_N]) {
+    for (int k = 0; k < AZ_N; k++) {
+        const double a = -PI + TWO_PI * (k + 0.5) / AZ_N;
+        tab[k].x = sin(a); tab[k].y = cos(a);
+    }
 }
 
 // Base.mod2pi for -2pi < v < 4pi without branches (the general formula with k = -1, 0, 1 and the same roundings);
@@ -1977,9 +1987,20 @@ __global__ void clone_gathered_kernel(unsigned char* buf, long long stride, Gath
     dst.down[o] = b[r]; dst.inj[o] = b[stride + r];
 }
 
-// End of the ion: fold the exact accumulators into the FP64 tally cells [c0, c1).  The words are first brought to their
-// unique form (0 <= word < 2^32 below the top one) so that the result is a function of the accumulated VALUE only, then
-// summed from the top down.
+// brings the words of a cell to their unique form: 0 <= word < 2^32 below the top one, which carries the sign
+__device__ __forceinline__ void acc_normalize(long long d[ACC_D]) {
+#pragma unroll
+    for (int k = 0; k + 1 < ACC_D; k++) {
+        const long long carry = d[k] >> 32;  // arithmetic shift = floor
+        d[k] -= carry << 32;
+        d[k + 1] += carry;
+    }
+}
+
+// End of the ion: fold the exact accumulators into the FP64 tally cells [c0, c1).  A cell becomes the correctly rounded
+// double of the integer its words hold, so the result is a function of the accumulated VALUE only: the magnitude's 64 bits
+// from the leading one down, with a sticky bit for everything below them, go through ONE round-to-nearest conversion and
+// are then scaled by a power of two (exact: every nonzero result is >= 2^ACC_ELO, far above the subnormals).
 __global__ void fold_accumulators_kernel(const long long* __restrict__ acc, size_t c0, size_t c1, double* tally) {
     const size_t c = c0 + (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= c1) return;
@@ -1988,16 +2009,29 @@ __global__ void fold_accumulators_kernel(const long long* __restrict__ acc, size
 #pragma unroll
     for (int k = 0; k < ACC_D; k++) { d[k] = acc[c * ACC_D + k]; any |= d[k] != 0; }
     if (!any) { tally[c] = 0.0; return; }
+    acc_normalize(d);
+    const bool neg = d[ACC_D - 1] < 0;
+    if (neg) {  // magnitude: negate word by word, then carry again
 #pragma unroll
-    for (int k = 0; k + 1 < ACC_D; k++) {
-        const long long carry = d[k] >> 32;  // arithmetic shift = floor
-        d[k] -= carry << 32;
-        d[k + 1] += carry;
+        for (int k = 0; k < ACC_D; k++) d[k] = -d[k];
+        acc_normalize(d);
     }
-    double v = 0.0;
+    // the magnitude as ACC_D + 1 digits of 32 bits (the top word holds up to 63)
+    uint32_t u[ACC_D + 1];
 #pragma unroll
-    for (int k = ACC_D - 1; k >= 0; k--) v = fma((double)d[k], scalbn(1.0, ACC_ELO + 32 * k), v);
-    tally[c] = v;
+    for (int k = 0; k < ACC_D; k++) u[k] = (uint32_t)d[k];
+    u[ACC_D] = (uint32_t)((unsigned long long)d[ACC_D - 1] >> 32);
+    int h = ACC_D;
+    while (h >= 0 && u[h] == 0) h--;
+    if (h < 0) { tally[c] = 0.0; return; }  // the adds cancelled exactly: +0
+    const int lz = __clz(u[h]);
+    const uint32_t u1 = h >= 1 ? u[h - 1] : 0u, u2 = h >= 2 ? u[h - 2] : 0u;
+    unsigned long long m = ((((unsigned long long)u[h] << 32) | u1) << lz) | ((unsigned long long)u2 >> (32 - lz));
+    bool sticky = (uint32_t)(u2 << lz) != 0u;
+    for (int k = 0; k + 2 < h; k++) sticky |= u[k] != 0u;
+    m |= sticky ? 1ull : 0ull;
+    const double v = scalbn(__ull2double_rn(m), ACC_ELO + 32 * (h - 1) - lz);
+    tally[c] = neg ? -v : v;
 }
 
 // particle_counter.jl:81-85: shock-frame dN(p) of the cosmic rays = sum of the PSD over the angle bins
