@@ -244,7 +244,7 @@ extern "C" int mcs_create(const McsConfig* cfg, McsHandle** out) {
     CUA(cudaMalloc(&h->d_l_save, (size_t)N)); CUA(cudaMalloc(&h->d_fate, (size_t)N * 4)); CUA(cudaMalloc(&h->d_helix, (size_t)N * 4));
     CUA(cudaMalloc(&h->d_retro, (size_t)N * 8)); CUA(cudaMalloc(&h->d_draws, (size_t)N * 8));
     CUA(cudaMalloc(&h->d_saved_idx, (size_t)N * 8));
-    const int scan_blocks = (int)((N + 1023) / 1024);
+    const long long scan_blocks = compaction_blocks(N);
     CUA(cudaMalloc(&h->d_block_cnt, (size_t)scan_blocks * 4)); CUA(cudaMalloc(&h->d_block_off, (size_t)scan_blocks * 8));
     CUA(cudaMalloc(&h->d_total, 8));
     // packed FP64 tally buffer
@@ -624,10 +624,7 @@ extern "C" int mcs_run_pcut(McsHandle* h, int32_t i_pcut, double pcut, double pc
 static int compact_saved(McsHandle* h) {
     const long long n = h->n_use;
     if (h->n_saved_last > 0) {
-        const int nb = (int)((n + 1023) / 1024);
-        count_saved_kernel<<<nb, 1024, 0, h->stream>>>(h->d_l_save, n, h->d_block_cnt);
-        scan_blocks_kernel<<<1, 1024, 0, h->stream>>>(h->d_block_cnt, nb, h->d_block_off, h->d_total);
-        compact_saved_kernel<<<nb, 1024, 0, h->stream>>>(h->d_l_save, n, h->d_block_off, h->d_saved_idx);
+        enqueue_compaction(h->d_l_save, n, h->d_block_cnt, h->d_block_off, h->d_total, h->d_saved_idx, h->stream);
         CU(cudaGetLastError());
         h->tm.other_launches += 3;
     }
@@ -681,22 +678,15 @@ extern "C" int mcs_split_explicit(McsHandle* h, int64_t i_mult, int64_t first_gl
 // the slices, the capacity check — comes out the same everywhere and no rank can leave the collective alone.
 static int split_multi_async(McsHandle* h, const long long* ns_all, int64_t n_pts_target, int64_t* n_new_local,
                              int64_t* n_new_global, int64_t* i_mult_out) {
-    GatherPrefix pre;
-    memset(&pre, 0, sizeof pre);
-    pre.nranks = h->nranks;
-    long long S = 0, max_ns = 0;
-    for (int r = 0; r < h->nranks; r++) { pre.start[r] = S; S += ns_all[r]; if (ns_all[r] > max_ns) max_ns = ns_all[r]; }
-    pre.start[h->nranks] = S;
-    h->n_saved_global_last = S;
-    if (S <= 0) return fail(MCS_ERR_STATE, "no saved particles to split");
-    long long i_mult = n_pts_target / S;  // cuts.jl:42 on the GLOBAL count
-    if (i_mult < 1) i_mult = 1;
-    const long long C = S * i_mult;
-    for (int r = 0; r < h->nranks; r++)  // the largest slice decides for everybody
-        if (C * (r + 1) / h->nranks - C * r / h->nranks > h->cfg.n_pts_max) return fail(MCS_ERR_ARG, "split population exceeds n_pts_max");
-    if (C > 0x100000000ll) return fail(MCS_ERR_ARG, "global particle index exceeds 2^32 (RNG counter width)");
-    const long long c0 = C * h->rank / h->nranks, c1 = C * (h->rank + 1) / h->nranks, n_out = c1 - c0;
-    const long long stride = (max_ns + 15) / 16 * 16;
+    SplitPlan plan;
+    const int pe = split_plan(ns_all, h->nranks, h->rank, n_pts_target, h->cfg.n_pts_max, &plan);
+    h->n_saved_global_last = plan.S;
+    if (pe == SPLIT_PLAN_BAD_RANKS) return fail(MCS_ERR_STATE, "bad rank/nranks");
+    if (pe == SPLIT_PLAN_NONE_SAVED) return fail(MCS_ERR_STATE, "no saved particles to split");
+    if (pe == SPLIT_PLAN_OVER_CAPACITY) return fail(MCS_ERR_ARG, "split population exceeds n_pts_max");
+    if (pe == SPLIT_PLAN_OVER_RANGE) return fail(MCS_ERR_ARG, "global particle index exceeds 2^32 (RNG counter width)");
+    const GatherPrefix& pre = plan.pre;
+    const long long i_mult = plan.i_mult, C = plan.C, c0 = plan.c0, n_out = plan.c1 - plan.c0, stride = plan.stride;
     if ((size_t)stride * 82 * (size_t)h->nranks > h->xchg_bytes) return fail(MCS_ERR_STATE, "split exchange buffer too small");
     CU(cudaEventRecord(h->ev2, h->stream));
     int rc = compact_saved(h);

@@ -18,6 +18,7 @@
 // FP64 scalar work with data-dependent control flow: no dense contraction, so no tensor cores / TMA.
 #pragma once
 #include <cstdint>
+#include <cstring>
 #include <cuda_runtime.h>
 
 #include "../../include/mcs.h"
@@ -1872,6 +1873,9 @@ __global__ void reduce_partials_kernel(const double* __restrict__ partials, int 
 
 // ---------------------------------------------------------------------------------------------
 // new_pcut (cuts.jl:34-98) on device: order-preserving compaction of l_save, then i_mult clones each.
+// COMPACT_TPB is the block size of all three compaction kernels (enqueue_compaction): one block count per COMPACT_TPB
+// particles, and the scan walks the counts in tiles of COMPACT_TPB.
+constexpr int COMPACT_TPB = 1024;
 __global__ void count_saved_kernel(const uint8_t* __restrict__ l_save, long long n, int* block_counts) {
     __shared__ int sh[32];
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1888,7 +1892,7 @@ __global__ void count_saved_kernel(const uint8_t* __restrict__ l_save, long long
 
 // single block: exclusive scan of block_counts (n_blocks entries) into block_offsets; total -> *total
 __global__ void scan_blocks_kernel(const int* __restrict__ counts, int n_blocks, long long* offsets, long long* total) {
-    __shared__ long long sh[1024];
+    __shared__ long long sh[COMPACT_TPB];
     __shared__ long long carry;
     if (threadIdx.x == 0) carry = 0;
     __syncthreads();
@@ -1923,6 +1927,21 @@ __global__ void compact_saved_kernel(const uint8_t* __restrict__ l_save, long lo
     int before = 0;
     for (int k = 0; k < w; k++) before += sh[k];
     if (v) saved_idx[offsets[blockIdx.x] + before + __popc(b & ((1u << lane) - 1u))] = i;
+}
+
+// entries of the block_cnt / block_off buffers that enqueue_compaction needs for n particles
+__host__ inline long long compaction_blocks(long long n) { return (n + COMPACT_TPB - 1) / COMPACT_TPB; }
+
+// The order-preserving compaction, enqueued on `stream` (n >= 1): saved_idx[0..*total) = the indices i < n with l_save[i]
+// set, in increasing order.  compact_saved_kernel reads offsets[blockIdx.x] under count_saved_kernel's block size, and the
+// scan's shared array holds one tile of COMPACT_TPB counts, so these launch shapes are fixed here and nowhere else.
+// Launch errors are left for the caller's cudaGetLastError.
+__host__ inline void enqueue_compaction(const uint8_t* l_save, long long n, int* block_cnt, long long* block_off,
+                                        long long* total, long long* saved_idx, cudaStream_t stream) {
+    const int nb = (int)compaction_blocks(n);
+    count_saved_kernel<<<nb, COMPACT_TPB, 0, stream>>>(l_save, n, block_cnt);
+    scan_blocks_kernel<<<1, COMPACT_TPB, 0, stream>>>(block_cnt, nb, block_off, total);
+    compact_saved_kernel<<<nb, COMPACT_TPB, 0, stream>>>(l_save, n, block_off, saved_idx);
 }
 
 // per-pcut exchange record of one rank, filled on the device so that the all-gather needs no host round trip first
@@ -1985,6 +2004,45 @@ __global__ void clone_gathered_kernel(unsigned char* buf, long long stride, Gath
     dst.grid[o] = g[r]; dst.tcut[o] = g[stride + r];
     const uint8_t* b = block + (size_t)stride * 80;
     dst.down[o] = b[r]; dst.inj[o] = b[stride + r];
+}
+
+// Host plan of the rebalancing split for one rank, from every rank's saved count ns_all[0..nranks): the prefix of the
+// gathered blocks, S saved in all, i_mult = max(target / S, 1) (cuts.jl:42 on the global count), C = S * i_mult children,
+// this rank's slice [c0, c1) = [C r / N, C (r + 1) / N) and the gather stride (the largest ns rounded up to 16 records).
+// Every rank computes the same plan but its slice, so all refuse together.  `pre` and S are filled on every path.
+struct SplitPlan {
+    GatherPrefix pre;
+    long long S, i_mult, C, c0, c1, stride;
+};
+enum SplitPlanError {
+    SPLIT_PLAN_OK = 0,
+    SPLIT_PLAN_BAD_RANKS,      // nranks outside 1..64 or rank outside 0..nranks-1
+    SPLIT_PLAN_NONE_SAVED,     // S == 0: nothing to split
+    SPLIT_PLAN_OVER_CAPACITY,  // the largest slice exceeds n_pts_max
+    SPLIT_PLAN_OVER_RANGE,     // C > 2^32: a child's global index would leave the RNG counter range
+};
+__host__ inline int split_plan(const long long* ns_all, int nranks, int rank, long long target, long long n_pts_max,
+                               SplitPlan* p) {
+    memset(p, 0, sizeof *p);
+    if (nranks < 1 || nranks > 64 || rank < 0 || rank >= nranks) return SPLIT_PLAN_BAD_RANKS;
+    p->pre.nranks = nranks;
+    long long S = 0, max_ns = 0;
+    for (int r = 0; r < nranks; r++) { p->pre.start[r] = S; S += ns_all[r]; if (ns_all[r] > max_ns) max_ns = ns_all[r]; }
+    p->pre.start[nranks] = S;
+    p->S = S;
+    if (S <= 0) return SPLIT_PLAN_NONE_SAVED;
+    long long i_mult = target / S;
+    if (i_mult < 1) i_mult = 1;
+    const long long C = S * i_mult;
+    for (int r = 0; r < nranks; r++)  // the largest slice decides for everybody
+        if (C * (r + 1) / nranks - C * r / nranks > n_pts_max) return SPLIT_PLAN_OVER_CAPACITY;
+    if (C > 0x100000000ll) return SPLIT_PLAN_OVER_RANGE;
+    p->i_mult = i_mult;
+    p->C = C;
+    p->c0 = C * rank / nranks;
+    p->c1 = C * (rank + 1) / nranks;
+    p->stride = (max_ns + 15) / 16 * 16;
+    return SPLIT_PLAN_OK;
 }
 
 // brings the words of a cell to their unique form: 0 <= word < 2^32 below the top one, which carries the sign

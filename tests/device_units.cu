@@ -40,7 +40,7 @@ __global__ void k_asin_bf(const double* x, long n, double* y) {
 
 // device buffers of one call, freed on every path out
 struct Bufs {
-    void* p[8] = {};
+    void* p[16] = {};
     int n = 0;
     cudaError_t err = cudaSuccess;
     template <class T> T* in(const T* h, size_t count) {
@@ -67,6 +67,19 @@ struct Bufs {
     }
     ~Bufs() { for (int i = 0; i < n; i++) cudaFree(p[i]); }
 };
+
+// A population of `cap` records held field by field in three arrays, as the split entry points take it from the host:
+// f64 = 8 fields x cap in PopPtrs order (weight, ptot, pb, x, xn_per, prp_x, acctime, phi), i64 = grid, tcut,
+// u8 = down, inj.  The view starts at record `first`.
+PopPtrs pop_view(double* f64, long long* i64, uint8_t* u8, long long cap, long long first) {
+    PopPtrs p;
+    memset(&p, 0, sizeof p);
+    double** f[8] = {&p.weight, &p.ptot, &p.pb, &p.x, &p.xn_per, &p.prp_x, &p.acctime, &p.phi};
+    for (int k = 0; k < 8; k++) *f[k] = f64 + k * cap + first;
+    p.grid = i64 + first; p.tcut = i64 + cap + first;
+    p.down = u8 + first; p.inj = u8 + cap + first;
+    return p;
+}
 
 }  // namespace
 
@@ -159,6 +172,128 @@ int du_asin_bf(const double* x, long n, int nr, double* y) {
     b.launched();
     b.out(y, d_y, n);
     return b.err;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// The split of new_pcut.  Populations cross in the field-major layout of pop_view.
+
+// enqueue_compaction on l_save[0..n): saved_idx gets all n entries (zero past *total)
+int du_compact(const uint8_t* l_save, long n, long long* saved_idx, long long* total) {
+    Bufs b;
+    const uint8_t* d_l = b.in(l_save, n);
+    const long long nb = compaction_blocks(n);
+    int* d_cnt = b.alloc<int>(nb);
+    long long* d_off = b.alloc<long long>(nb);
+    long long* d_total = b.alloc<long long>(1);
+    long long* d_idx = b.alloc<long long>(n);
+    if (b.err) return b.err;
+    if (n > 0) enqueue_compaction(d_l, n, d_cnt, d_off, d_total, d_idx, 0);
+    b.launched();
+    b.out(total, d_total, 1);
+    b.out(saved_idx, d_idx, n);
+    return b.err;
+}
+
+// the single-rank split (the library's split_local_async): compaction, then clone_kernel into n_out = *total * i_mult
+// children; fails with cudaErrorInvalidValue if they do not fit in `cap` records
+int du_split_local(const double* f64, const long long* i64, const uint8_t* u8, const uint8_t* l_save, long n, long i_mult,
+                   long cap, double* out_f64, long long* out_i64, uint8_t* out_u8, long long* total) {
+    if (i_mult < 1) return cudaErrorInvalidValue;
+    Bufs b;
+    double* d_f = b.in(f64, 8 * (size_t)n);
+    long long* d_i = b.in(i64, 2 * (size_t)n);
+    uint8_t* d_u = b.in(u8, 2 * (size_t)n);
+    const uint8_t* d_l = b.in(l_save, n);
+    const long long nb = compaction_blocks(n);
+    int* d_cnt = b.alloc<int>(nb);
+    long long* d_off = b.alloc<long long>(nb);
+    long long* d_total = b.alloc<long long>(1);
+    long long* d_idx = b.alloc<long long>(n);
+    double* o_f = b.alloc<double>(8 * (size_t)cap);
+    long long* o_i = b.alloc<long long>(2 * (size_t)cap);
+    uint8_t* o_u = b.alloc<uint8_t>(2 * (size_t)cap);
+    if (b.err) return b.err;
+    if (n > 0) enqueue_compaction(d_l, n, d_cnt, d_off, d_total, d_idx, 0);
+    b.launched();
+    b.out(total, d_total, 1);
+    if (b.err) return b.err;
+    const long long n_out = *total * i_mult;
+    if (n_out > cap) return cudaErrorInvalidValue;
+    if (n_out > 0)
+        clone_kernel<<<blocks(n_out), TPB>>>(pop_view(d_f, d_i, d_u, n, 0), pop_view(o_f, o_i, o_u, cap, 0), d_idx, n_out, i_mult);
+    b.launched();
+    b.out(out_f64, o_f, 8 * (size_t)cap); b.out(out_i64, o_i, 2 * (size_t)cap); b.out(out_u8, o_u, 2 * (size_t)cap);
+    return b.err;
+}
+
+// The rebalancing split (the library's split_multi_async) of `nranks` ranks emulated on one device; rank q holds records
+// [first_q, first_q + n_per_rank[q]) of the concatenated population.  Each rank compacts its own l_save, which gives
+// ns_all, and plans with split_plan; rank q packs its saved records into block q of one exchange buffer, which is then
+// byte for byte what the all-gather leaves on every rank; then every rank clones its slice [c0, c1) of the global child
+// range out of it.  The slices land at records [c0, c1) of the output (cap records), n_out[r] = c1 - c0.  A refused plan
+// or C > cap gives cudaErrorInvalidValue.
+int du_split_ranks(int nranks, const long long* n_per_rank, const uint8_t* l_save, const double* f64, const long long* i64,
+                   const uint8_t* u8, long long target, long long n_pts_max, long cap, double* out_f64, long long* out_i64,
+                   uint8_t* out_u8, long long* n_out, long long* i_mult) {
+    if (nranks < 1 || nranks > 64) return cudaErrorInvalidValue;
+    long long first[65] = {0}, nb_max = 1;
+    for (int q = 0; q < nranks; q++) {
+        first[q + 1] = first[q] + n_per_rank[q];
+        if (compaction_blocks(n_per_rank[q]) > nb_max) nb_max = compaction_blocks(n_per_rank[q]);
+    }
+    const long long N = first[nranks];
+    Bufs b;
+    double* d_f = b.in(f64, 8 * (size_t)N);
+    long long* d_i = b.in(i64, 2 * (size_t)N);
+    uint8_t* d_u = b.in(u8, 2 * (size_t)N);
+    const uint8_t* d_l = b.in(l_save, N);
+    int* d_cnt = b.alloc<int>(nb_max);
+    long long* d_off = b.alloc<long long>(nb_max);
+    long long* d_total = b.alloc<long long>(nranks);
+    long long* d_idx = b.alloc<long long>(N);
+    if (b.err) return b.err;
+    for (int q = 0; q < nranks; q++)
+        if (n_per_rank[q] > 0) enqueue_compaction(d_l + first[q], n_per_rank[q], d_cnt, d_off, d_total + q, d_idx + first[q], 0);
+    b.launched();
+    long long ns_all[64];
+    b.out(ns_all, d_total, nranks);
+    if (b.err) return b.err;
+    SplitPlan plan[64];
+    for (int r = 0; r < nranks; r++)
+        if (split_plan(ns_all, nranks, r, target, n_pts_max, &plan[r]) != SPLIT_PLAN_OK) return cudaErrorInvalidValue;
+    const long long stride = plan[0].stride;
+    if (plan[0].C > cap) return cudaErrorInvalidValue;
+    unsigned char* d_x = b.alloc<unsigned char>((size_t)nranks * (size_t)stride * 82);
+    double* o_f = b.alloc<double>(8 * (size_t)cap);
+    long long* o_i = b.alloc<long long>(2 * (size_t)cap);
+    uint8_t* o_u = b.alloc<uint8_t>(2 * (size_t)cap);
+    if (b.err) return b.err;
+    for (int q = 0; q < nranks; q++)
+        if (ns_all[q] > 0)
+            pack_saved_kernel<<<blocks(ns_all[q]), TPB>>>(pop_view(d_f, d_i, d_u, N, first[q]), d_idx + first[q], ns_all[q],
+                                                          d_x + (size_t)q * (size_t)stride * 82, stride);
+    for (int r = 0; r < nranks; r++) {
+        n_out[r] = plan[r].c1 - plan[r].c0;
+        if (n_out[r] > 0)
+            clone_gathered_kernel<<<blocks(n_out[r]), TPB>>>(d_x, stride, plan[r].pre, pop_view(o_f, o_i, o_u, cap, plan[r].c0),
+                                                             plan[r].c0, n_out[r], plan[r].i_mult);
+    }
+    b.launched();
+    b.out(out_f64, o_f, 8 * (size_t)cap); b.out(out_i64, o_i, 2 * (size_t)cap); b.out(out_u8, o_u, 2 * (size_t)cap);
+    *i_mult = plan[0].i_mult;
+    return b.err;
+}
+
+// split_plan alone (host code, no device needed): returns its SplitPlanError; out = {S, i_mult, C, c0, c1, stride},
+// start = the gather prefix start[0..nranks]
+int du_split_plan(const long long* ns_all, int nranks, int rank, long long target, long long n_pts_max, long long* out,
+                  long long* start) {
+    SplitPlan p;
+    const int rc = split_plan(ns_all, nranks, rank, target, n_pts_max, &p);
+    const long long v[6] = {p.S, p.i_mult, p.C, p.c0, p.c1, p.stride};
+    memcpy(out, v, sizeof v);
+    if (p.pre.nranks > 0) memcpy(start, p.pre.start, (size_t)(p.pre.nranks + 1) * sizeof(long long));
+    return rc;
 }
 
 }  // extern "C"

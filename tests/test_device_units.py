@@ -4,7 +4,9 @@ tests/device_units.cu includes csrc/mcs_device.cuh and is built with the library
 so each kernel here runs the code the library inlines.  References are exact: integer / Fraction arithmetic for the exact
 tally accumulators (acc_add + fold_accumulators_kernel), mpmath at 60 digits for the fast loop's math (az_sincos,
 rsqrt_nr) and for the device build of the shared sincos_bf / asin_bf (tests/test_device_math.py holds their host build to
-libm).  Run with -s to see the worst error measured for each primitive.
+libm), numpy index arithmetic and bit patterns for the split of new_pcut (enqueue_compaction, clone_kernel, and the
+rebalancing split — split_plan, pack_saved_kernel, clone_gathered_kernel — of up to 64 ranks emulated on one device).
+Run with -s to see the worst error measured for each primitive.
 """
 import ctypes as C
 import math
@@ -23,6 +25,7 @@ SIN_UPPER_LIMIT = np.nextafter(1.0, 0.0)
 P_D = C.POINTER(C.c_double)
 P_I64 = C.POINTER(C.c_int64)
 P_U32 = C.POINTER(C.c_uint32)
+P_U8 = C.POINTER(C.c_uint8)
 
 
 @pytest.fixture(scope="module")
@@ -40,6 +43,11 @@ def harness(tmp_path_factory):
     lib.du_roots.argtypes = [P_D, C.c_long, P_D, P_D, P_D]
     lib.du_sincos_bf.argtypes = [P_D, C.c_long, P_D, P_D]
     lib.du_asin_bf.argtypes = [P_D, C.c_long, C.c_int, P_D]
+    lib.du_compact.argtypes = [P_U8, C.c_long, P_I64, P_I64]
+    lib.du_split_local.argtypes = [P_D, P_I64, P_U8, P_U8, C.c_long, C.c_long, C.c_long, P_D, P_I64, P_U8, P_I64]
+    lib.du_split_ranks.argtypes = [C.c_int, P_I64, P_U8, P_D, P_I64, P_U8, C.c_longlong, C.c_longlong, C.c_long, P_D, P_I64,
+                                   P_U8, P_I64, P_I64]
+    lib.du_split_plan.argtypes = [P_I64, C.c_int, C.c_int, C.c_longlong, C.c_longlong, P_I64, P_I64]
     return lib
 
 
@@ -412,3 +420,254 @@ def test_asin_bf_device_build(harness, nr):
     h = x.size // 2
     assert np.array_equal(y[h:].view(np.int64), (-y[:h]).view(np.int64))
     assert np.array_equal(y[~nz].view(np.int64), x[~nz].view(np.int64))
+
+
+# ----------------------------------------------------------------------------------------------------------------------
+# The split of new_pcut (cuts.jl:69-91): child o of a split is the saved parent flatnonzero(l_save)[o // i_mult] with every
+# field copied and its weight w / i_mult (one IEEE division).  compaction_blocks tiles the particles by 1024 and the scan
+# carries its running total from one tile of 1024 block counts (2^20 particles) to the next, so the sizes below straddle
+# both boundaries.  Populations cross in the harness's field-major layout: f64 [8, n] (weight first), i64 [2, n], u8 [2, n].
+
+SPLIT_PLAN_OK, SPLIT_PLAN_BAD_RANKS, SPLIT_PLAN_NONE_SAVED, SPLIT_PLAN_OVER_CAPACITY, SPLIT_PLAN_OVER_RANGE = range(5)
+COMPACTION_SIZES = [1, 31, 32, 33, 1023, 1024, 1025, 2**20 - 1, 2**20, 2**20 + 1, 2**20 + 1024, 10_000_019, 3 * 2**24 + 5]
+
+
+def _save_patterns(n, rng):
+    """name -> l_save of n particles."""
+    def one_at(*i):
+        return np.bincount(np.concatenate([np.atleast_1d(np.asarray(x, np.int64)) for x in i]), minlength=n).astype(np.uint8)
+    edges = np.arange(1024, n, 1024)  # every 2^20 boundary is one of these
+    return {"all": np.ones(n, np.uint8), "first": one_at(0), "last": one_at(n - 1),
+            "block_edges": one_at(0, edges - 1, edges),
+            "every_other": (np.arange(n) % 2 == 0).astype(np.uint8),
+            "sparse": (rng.random(n) < 1e-4).astype(np.uint8), "half": (rng.random(n) < 0.5).astype(np.uint8)}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n", COMPACTION_SIZES)
+def test_compaction(harness, n):
+    """enqueue_compaction against np.flatnonzero, for every pattern: the saved indices in order, the count, and nothing
+    written past it.  3 * 2^24 + 5 particles make 49 scan tiles, the last of them holding a single block count."""
+    rng = np.random.default_rng(31 + n % 1000)
+    for name, l_save in _save_patterns(n, rng).items():
+        idx, total = np.zeros(n, np.int64), np.zeros(1, np.int64)
+        _ok(harness.du_compact(_p(l_save, P_U8), n, _p(idx, P_I64), _p(total, P_I64)))
+        want = np.flatnonzero(l_save)
+        assert total[0] == want.size, f"n = {n}, {name}: total {total[0]} != {want.size}"
+        bad = np.flatnonzero(idx[:want.size] != want)
+        assert bad.size == 0, f"n = {n}, {name}: {bad.size} saved indices wrong, first at output {bad[0]}"
+        assert not idx[want.size:].any(), f"n = {n}, {name}: written past the count"
+
+
+def _random_pop(rng, n):
+    """A population whose 12 fields are random bit patterns: any finite double (subnormals, -0 included), any int64, any
+    byte."""
+    bits = rng.integers(0, 2**64, (8, n), dtype=np.uint64)
+    top = np.uint64(0x7FF) << np.uint64(52)
+    bits[(bits & top) == top] ^= np.uint64(1) << np.uint64(62)  # exponent all ones (inf / NaN) -> finite
+    return (bits.view(np.float64), rng.integers(-(2**63), 2**63 - 1, (2, n), dtype=np.int64, endpoint=True),
+            rng.integers(0, 256, (2, n), dtype=np.uint8, endpoint=False))
+
+
+def _ref_split(f64, i64, u8, l_save, i_mult):
+    """The split in cuts.jl:69-91 order: children of the k-th saved particle at rows [k i_mult, (k + 1) i_mult)."""
+    par = np.repeat(np.flatnonzero(l_save), i_mult)
+    f = f64[:, par]
+    f[0] = f[0] / np.float64(i_mult)
+    return f, i64[:, par], u8[:, par]
+
+
+def _assert_pop_equal(got, want, what):
+    for a, b, nm in zip(got, want, ("f64", "i64", "u8")):
+        a = a.view(np.int64) if a.dtype == np.float64 else a
+        b = b.view(np.int64) if b.dtype == np.float64 else b
+        assert a.shape == b.shape, f"{what}: {nm} shape {a.shape} != {b.shape}"
+        bad = np.argwhere(a != b)
+        assert bad.size == 0, f"{what}: {len(bad)} {nm} values differ, first (field, child) = {tuple(bad[0])}"
+
+
+def _split_local(lib, pop, l_save, i_mult):
+    f64, i64, u8 = (np.ascontiguousarray(a) for a in pop)
+    n, cap = len(l_save), int(l_save.sum()) * i_mult
+    out = (np.zeros((8, cap)), np.zeros((2, cap), np.int64), np.zeros((2, cap), np.uint8))
+    total = np.zeros(1, np.int64)
+    _ok(lib.du_split_local(_p(f64), _p(i64, P_I64), _p(u8, P_U8), _p(l_save, P_U8), n, i_mult, cap, _p(out[0]),
+                           _p(out[1], P_I64), _p(out[2], P_U8), _p(total, P_I64)))
+    assert total[0] == l_save.sum()
+    return out
+
+
+@pytest.mark.gpu
+def test_split_local(harness):
+    """Compaction + clone_kernel (the single-rank split) bit for bit against the reference split, for i_mult 1, 3, 1000
+    and target // ns, on populations of random bit patterns, two of them past one scan tile (2^20 particles)."""
+    rng = np.random.default_rng(32)
+    cases = [(5000, 0.3, 1), (5000, 0.3, 3), (5000, 0.3, 1000), (4099, 0.05, "target"),
+             (2**20 + 4097, 0.5, "target"), (3_000_017, 0.01, "target")]
+    for n, density, i_mult in cases:
+        pop, l_save = _random_pop(rng, n), (rng.random(n) < density).astype(np.uint8)
+        if i_mult == "target":
+            i_mult = max(4_000_000 // int(l_save.sum()), 1)
+        _assert_pop_equal(_split_local(harness, pop, l_save, i_mult), _ref_split(*pop, l_save, i_mult),
+                          f"n = {n}, i_mult = {i_mult}")
+
+
+def _rank_case(rng, sizes, density, target, n_pts_max=None):
+    """Ranks of the given population sizes; density[q] = fraction of rank q's particles saved."""
+    l_save = [(rng.random(s) < d).astype(np.uint8) for s, d in zip(sizes, density)]
+    return dict(sizes=np.asarray(sizes, np.int64), l_save=l_save, target=target, n_pts_max=n_pts_max or 2**31 - 1)
+
+
+def _rank_cases():
+    rng = np.random.default_rng(33)
+    r8 = rng.integers(0, 5000, 8)
+    r64 = rng.integers(0, 3000, 64)
+    d64 = np.where(np.arange(64) % 7 == 3, 0.0, rng.uniform(0.05, 0.9, 64))
+    one_of_64 = np.where(np.arange(64) == 41, 0.3, 0.0)
+    r8_one, r64_one = np.where(np.arange(8) == 5, 3001, r8), np.where(np.arange(64) == 41, 2999, r64)
+    return {
+        "1 rank": _rank_case(rng, [777], [0.4], 10_000),
+        "2 ranks, first empty": _rank_case(rng, [1000, 3001], [0.0, 0.3], 50_000),
+        "2 ranks, target below S": _rank_case(rng, [2047, 1500], [0.7, 0.6], 1000),
+        "3 ranks, middle empty": _rank_case(rng, [513, 0, 2049], [0.5, 0.5, 0.5], 100_000),
+        "3 ranks, middle saves none": _rank_case(rng, [1111, 2222, 333], [0.3, 0.0, 0.9], 7),
+        "3 ranks past one scan tile": _rank_case(rng, [2**20 + 5, 17, 2**21 - 3], [0.5, 1.0, 0.25], 2_000_000),
+        "8 ranks, last empty": _rank_case(rng, r8, [0.4] * 7 + [0.0], 100_003),
+        "8 ranks, all but one empty": _rank_case(rng, r8_one, [0.0] * 5 + [0.5] + [0.0] * 2, 12_345),
+        "64 ranks": _rank_case(rng, r64, d64, 1_000_003),
+        "64 ranks, all but one empty": _rank_case(rng, r64_one, one_of_64, 99_999),
+        "64 ranks, target below S": _rank_case(rng, r64, rng.uniform(0, 1, 64), 10),
+    }
+
+
+def _split_ranks(lib, case, pop, l_save):
+    sizes, nr = case["sizes"], len(case["sizes"])
+    f64, i64, u8 = (np.ascontiguousarray(a) for a in pop)
+    S = int(l_save.sum())
+    C_ = S * max(case["target"] // S, 1)
+    out = (np.zeros((8, C_)), np.zeros((2, C_), np.int64), np.zeros((2, C_), np.uint8))
+    n_out, i_mult = np.zeros(nr, np.int64), np.zeros(1, np.int64)
+    _ok(lib.du_split_ranks(nr, _p(sizes, P_I64), _p(l_save, P_U8), _p(f64), _p(i64, P_I64), _p(u8, P_U8), case["target"],
+                           case["n_pts_max"], C_, _p(out[0]), _p(out[1], P_I64), _p(out[2], P_U8), _p(n_out, P_I64),
+                           _p(i_mult, P_I64)))
+    return out, n_out, int(i_mult[0])
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", list(_rank_cases()))
+def test_split_emulated_ranks(harness, name):
+    """The rebalancing split of N ranks emulated on one device (split_plan, pack_saved_kernel into the exchange buffer as
+    the all-gather leaves it, clone_gathered_kernel per rank): rank r's slice is rows [C r / N, C (r + 1) / N) of the
+    reference split of the concatenated population, bit for bit, and the slices together are what one rank computes
+    (du_split_local on the concatenated population)."""
+    case = _rank_cases()[name]
+    rng = np.random.default_rng(34)
+    sizes, nr = case["sizes"], len(case["sizes"])
+    l_save = np.concatenate(case["l_save"])
+    pop = _random_pop(rng, int(sizes.sum()))
+    ns = np.array([int(x.sum()) for x in case["l_save"]])
+    S = int(ns.sum())
+    i_mult_ref = max(case["target"] // S, 1)
+    C_ = S * i_mult_ref
+    out, n_out, i_mult = _split_ranks(harness, case, pop, l_save)
+    assert i_mult == i_mult_ref
+    ref = _ref_split(*pop, l_save, i_mult_ref)
+    for r in range(nr):
+        c0, c1 = C_ * r // nr, C_ * (r + 1) // nr
+        assert n_out[r] == c1 - c0, f"{name}: rank {r} got {n_out[r]} children, not {c1 - c0}"
+        _assert_pop_equal(tuple(a[:, c0:c1] for a in out), tuple(a[:, c0:c1] for a in ref), f"{name}, rank {r}")
+    _assert_pop_equal(out, _split_local(harness, pop, l_save, i_mult_ref), f"{name}: N ranks against one")
+    print(f"\n{name}: ns {ns.min()}..{ns.max()} over {nr} ranks, S = {S}, i_mult = {i_mult}, C = {C_}, C % N = {C_ % nr}, "
+          f"max ns % 16 = {ns.max() % 16}")
+
+
+def test_emulated_rank_cases_cover_the_edges():
+    """The cases above hold every edge of the plan: ranks saving nothing first, last, in the middle and all but one; the
+    largest ns not a multiple of 16 (padded stride); a target below S (i_mult clamped to 1); C not divisible by N."""
+    seen = set()
+    for case in _rank_cases().values():
+        ns = np.array([int(x.sum()) for x in case["l_save"]])
+        S, nr = int(ns.sum()), len(ns)
+        C_ = S * max(case["target"] // S, 1)
+        seen |= {k for k, v in {"first empty": ns[0] == 0 and nr > 1, "last empty": ns[-1] == 0 and nr > 1,
+                                "middle empty": nr > 2 and (ns[1:-1] == 0).any(), "all but one": nr > 2 and (ns > 0).sum() == 1,
+                                "padded stride": ns.max() % 16 != 0, "clamped": case["target"] < S,
+                                "ragged slices": C_ % nr != 0}.items() if v}
+        for n in (1, 2, 3, 8, 64):
+            if nr == n:
+                seen.add(n)
+    assert seen == {"first empty", "last empty", "middle empty", "all but one", "padded stride", "clamped", "ragged slices",
+                    1, 2, 3, 8, 64}, seen
+
+
+def _plan(lib, ns_all, rank, target, n_pts_max):
+    ns_all = np.ascontiguousarray(ns_all, dtype=np.int64)
+    out, start = np.full(6, -1, np.int64), np.zeros(65, np.int64)
+    rc = lib.du_split_plan(_p(ns_all, P_I64), len(ns_all), rank, target, n_pts_max, _p(out, P_I64), _p(start, P_I64))
+    return rc, dict(zip(("S", "i_mult", "C", "c0", "c1", "stride"), (int(v) for v in out))), start[:len(ns_all) + 1]
+
+
+def test_split_plan_formula(harness):
+    """split_plan (host code, no GPU) over a sweep of (S, N, target): i_mult = max(target // S, 1), C = S i_mult, rank r's
+    slice [C r // N, C (r + 1) // N), stride = largest ns rounded up to 16, the gather prefix the running sum of ns_all."""
+    rng = np.random.default_rng(35)
+    n_cases = 0
+    for nr in (1, 2, 3, 5, 8, 17, 63, 64):
+        for _ in range(40):
+            ns_all = rng.integers(0, int(rng.choice([2, 100, 10**5, 10**7])), nr)
+            ns_all[rng.random(nr) < 0.3] = 0
+            S = int(ns_all.sum())
+            if S == 0:
+                ns_all[rng.integers(0, nr)] = 1
+                S = 1
+            target = int(rng.choice([0, 1, S - 1, S, S + 1, 2 * S - 1, int(rng.integers(0, 10**9))]))
+            i_mult = max(target // S, 1)
+            C_ = S * i_mult
+            if C_ > 2**32:
+                continue
+            for r in range(nr):
+                rc, p, start = _plan(harness, ns_all, r, target, 2**62)
+                assert rc == SPLIT_PLAN_OK
+                assert p == {"S": S, "i_mult": i_mult, "C": C_, "c0": C_ * r // nr, "c1": C_ * (r + 1) // nr,
+                             "stride": -(-int(ns_all.max()) // 16) * 16}, (ns_all, r, target)
+                assert np.array_equal(start, np.concatenate([[0], np.cumsum(ns_all)]))
+            n_cases += 1
+    assert n_cases > 250
+
+
+def test_split_plan_refusals(harness):
+    """The refusals at their exact edges: the largest slice at n_pts_max is taken and at n_pts_max + 1 refused; C = 2^32 is
+    taken and C = 2^32 + 1 refused (saved counts with no memory behind them); S = 0 and a bad rank layout are refused.
+    A refused plan still reports S (the library keeps it as the ion's global saved count)."""
+    rng = np.random.default_rng(36)
+    for _ in range(300):
+        nr = int(rng.choice([1, 2, 3, 7, 64]))
+        ns_all = rng.integers(0, 1000, nr)
+        ns_all[0] += 1
+        S = int(ns_all.sum())
+        target = int(rng.integers(0, 10**6))
+        C_ = S * max(target // S, 1)
+        largest = max(C_ * (r + 1) // nr - C_ * r // nr for r in range(nr))
+        for r in {0, nr - 1}:
+            assert _plan(harness, ns_all, r, target, largest)[0] == SPLIT_PLAN_OK
+            rc, p, _ = _plan(harness, ns_all, r, target, largest - 1)
+            assert rc == SPLIT_PLAN_OVER_CAPACITY and p["S"] == S
+    big = 2**62
+    for ns_all, target, want in (([2**31, 2**31], 0, SPLIT_PLAN_OK), ([2**31, 2**31 + 1], 0, SPLIT_PLAN_OVER_RANGE),
+                                 ([2**32], 2**32, SPLIT_PLAN_OK), ([2**32 + 1], 0, SPLIT_PLAN_OVER_RANGE),
+                                 ([2**16], 2**32, SPLIT_PLAN_OK), ([2**16], 2**32 + 2**16, SPLIT_PLAN_OVER_RANGE),
+                                 ([1, 2**16 - 1], 2**32 + 2**16 - 1, SPLIT_PLAN_OK),
+                                 ([3] * 63 + [2**32 + 1 - 189], 0, SPLIT_PLAN_OVER_RANGE),
+                                 ([3] * 63 + [2**32 - 189], 5, SPLIT_PLAN_OK)):
+        rc, p, _ = _plan(harness, ns_all, len(ns_all) - 1, target, big)
+        assert rc == want, (ns_all[-3:], target, rc)
+        if want == SPLIT_PLAN_OK:
+            assert p["C"] == 2**32 and p["c1"] == 2**32
+    # the capacity check comes first: at C = 2^32 + 1 on one rank with n_pts_max = C - 1 it is the capacity that refuses
+    assert _plan(harness, [2**32 + 1], 0, 0, 2**32)[0] == SPLIT_PLAN_OVER_CAPACITY
+    for nr in (1, 2, 64):
+        rc, p, start = _plan(harness, [0] * nr, nr - 1, 10**6, big)
+        assert rc == SPLIT_PLAN_NONE_SAVED and p["S"] == 0 and not start.any()
+    assert _plan(harness, [1, 1], 2, 10, big)[0] == SPLIT_PLAN_BAD_RANKS
+    assert _plan(harness, [1, 1], -1, 10, big)[0] == SPLIT_PLAN_BAD_RANKS
+    assert _plan(harness, [1] * 65, 0, 10, big)[0] == SPLIT_PLAN_BAD_RANKS
