@@ -107,7 +107,8 @@ struct McsHandle {
     double* d_boost = nullptr; // 3 arrays of (ng+2): ux/ut, uz/ut, ux*uz/ut^2
     double* d_grid = nullptr;  // 10 arrays of (ng+2): xg ux uz ut gsf gef bt sinth costh (bef unused) + tcuts(NA_C)
     double* d_zone = nullptr;  // eps_target, recv_pool [ng] each
-    PopPtrs pop[3];            // cur, saved, next
+    unsigned char* d_pop = nullptr;  // the three population blocks, one after the other
+    PopPtrs pop[3];            // views of them: cur, saved, next
     int cur = 0, nxt = 2;      // saved is always pop[1]
     uint8_t* d_l_save = nullptr;
     int *d_fate = nullptr, *d_helix = nullptr;
@@ -152,20 +153,6 @@ struct McsHandle {
 
 static int check_index_range(long long first_global, long long n);
 
-static int pop_alloc(PopPtrs& p, long long n) {
-    size_t nd = (size_t)n;
-    CU(cudaMalloc(&p.weight, nd * 8)); CU(cudaMalloc(&p.ptot, nd * 8)); CU(cudaMalloc(&p.pb, nd * 8));
-    CU(cudaMalloc(&p.x, nd * 8)); CU(cudaMalloc(&p.xn_per, nd * 8)); CU(cudaMalloc(&p.prp_x, nd * 8));
-    CU(cudaMalloc(&p.acctime, nd * 8)); CU(cudaMalloc(&p.phi, nd * 8)); CU(cudaMalloc(&p.grid, nd * 8));
-    CU(cudaMalloc(&p.tcut, nd * 8)); CU(cudaMalloc(&p.down, nd)); CU(cudaMalloc(&p.inj, nd));
-    return MCS_OK;
-}
-static void pop_free(PopPtrs& p) {
-    cudaFree(p.weight); cudaFree(p.ptot); cudaFree(p.pb); cudaFree(p.x); cudaFree(p.xn_per); cudaFree(p.prp_x);
-    cudaFree(p.acctime); cudaFree(p.phi); cudaFree(p.grid); cudaFree(p.tcut); cudaFree(p.down); cudaFree(p.inj);
-    memset(&p, 0, sizeof p);
-}
-
 static size_t psd_len(const McsHandle* h) { return (size_t)(h->M + 2) * (size_t)(h->T + 2) * (size_t)h->ng; }
 
 extern "C" int mcs_destroy(McsHandle* h) {
@@ -174,8 +161,7 @@ extern "C" int mcs_destroy(McsHandle* h) {
     if (h->stream) cudaStreamSynchronize(h->stream);
     if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
     cudaFree(h->d_grid); cudaFree(h->d_boost); cudaFree(h->d_zone); cudaFree(h->d_az);
-    for (auto& p : h->pop) pop_free(p);
-    cudaFree(h->d_l_save); cudaFree(h->d_fate); cudaFree(h->d_helix); cudaFree(h->d_retro); cudaFree(h->d_draws);
+    cudaFree(h->d_pop); cudaFree(h->d_l_save); cudaFree(h->d_fate); cudaFree(h->d_helix); cudaFree(h->d_retro); cudaFree(h->d_draws);
     cudaFree(h->d_saved_idx); cudaFree(h->d_block_off); cudaFree(h->d_total); cudaFree(h->d_block_cnt);
     cudaFree(h->d_tally); cudaFree(h->d_acc); cudaFree(h->d_u64); cudaFree(h->d_tg); cudaFree(h->d_tpx); cudaFree(h->d_tpt); cudaFree(h->d_tw);
     cudaFree(h->d_inj); cudaFree(h->d_partials); cudaFree(h->d_replay_u); cudaFree(h->d_replay_off); cudaFree(h->d_trace_slot);
@@ -229,8 +215,6 @@ extern "C" int mcs_create(const McsConfig* cfg, McsHandle** out) {
     if (h->block > MCS_BLOCK || h->block < 32 || (h->block & 31)) h->block = MCS_BLOCK;
     h->blocks_per_sm = env_int("MCS_BLOCKS_PER_SM", MCS_MIN_BLOCKS);
     h->max_blocks = h->n_sm * h->blocks_per_sm;
-    int rc = MCS_OK;
-#define TRY(x) do { rc = (x); if (rc != MCS_OK) { mcs_destroy(h); return rc; } } while (0)
 #define CUA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { fail(MCS_ERR_NOMEM, "CUDA alloc: %s at %s", cudaGetErrorString(e_), #call); mcs_destroy(h); return MCS_ERR_NOMEM; } } while (0)
     CUA(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
     CUA(cudaEventCreate(&h->ev0)); CUA(cudaEventCreate(&h->ev1)); CUA(cudaEventCreate(&h->ev2)); CUA(cudaEventCreate(&h->ev3)); CUA(cudaEventCreate(&h->ev4)); CUA(cudaEventCreate(&h->ev5));
@@ -240,7 +224,9 @@ extern "C" int mcs_create(const McsConfig* cfg, McsHandle** out) {
     CUA(cudaMalloc(&h->d_boost, (size_t)3 * ng2 * 8));
     CUA(cudaMalloc(&h->d_zone, (size_t)2 * ng * 8));
     CUA(cudaMalloc(&h->d_az, (size_t)AZ_N * sizeof(double2)));
-    for (auto& p : h->pop) TRY(pop_alloc(p, N));
+    const long long cap = pop_cap(N);
+    CUA(cudaMalloc(&h->d_pop, (size_t)3 * (size_t)cap * POP_REC_BYTES));
+    for (int k = 0; k < 3; k++) h->pop[k] = pop_view(h->d_pop + (size_t)k * (size_t)cap * POP_REC_BYTES, cap, 0);
     CUA(cudaMalloc(&h->d_l_save, (size_t)N)); CUA(cudaMalloc(&h->d_fate, (size_t)N * 4)); CUA(cudaMalloc(&h->d_helix, (size_t)N * 4));
     CUA(cudaMalloc(&h->d_retro, (size_t)N * 8)); CUA(cudaMalloc(&h->d_draws, (size_t)N * 8));
     CUA(cudaMalloc(&h->d_saved_idx, (size_t)N * 8));
@@ -268,7 +254,6 @@ extern "C" int mcs_create(const McsConfig* cfg, McsHandle** out) {
     // large grids: fewer warps per block so that the per-warp flux partials still fit (the per-launch shared-memory
     // attribute is set in mcs_run_pcut: it belongs to the function and the device, not to this handle)
     while (h->block > 32 && block_smem_bytes(ng, h->block / 32) > (size_t)200 * 1024 / (size_t)h->blocks_per_sm) h->block /= 2;
-#undef TRY
 #undef CUA
     // static part of the kernel parameters
     DevParams& P = h->P;
@@ -358,8 +343,7 @@ extern "C" int mcs_comm_init(McsHandle* h, int rank, int nranks, const void* id1
     // Exchange buffer of the rebalancing split, sized for the worst case (every rank saves its whole population) here,
     // where a failure is reported to each caller before any collective: inside the pcut loop a rank that bailed out
     // alone would leave the others blocked in the next all-gather.
-    const size_t stride_max = ((size_t)h->cfg.n_pts_max + 15) / 16 * 16;
-    const size_t need = stride_max * 82 * (size_t)nranks;
+    const size_t need = (size_t)pop_cap(h->cfg.n_pts_max) * POP_REC_BYTES * (size_t)nranks;
     cudaFree(h->d_xchg); h->d_xchg = nullptr; h->xchg_bytes = 0;
     if (cudaMalloc(&h->d_xchg, need) != cudaSuccess) return fail(MCS_ERR_NOMEM, "cannot allocate the split exchange buffer");
     h->xchg_bytes = need;
@@ -399,6 +383,31 @@ extern "C" int mcs_set_profile(McsHandle* h, int32_t n_grid, const double* xg, c
     return MCS_OK;
 }
 
+// The start of an ion, shared by mcs_begin_ion and mcs_begin_ion_generate: resets the handle's ion state, clears the
+// tallies (clear_psd!, ion_init.jl:1-16) and every other per-ion sum, then runs `setup`, which fills the current population
+// with its n particles.  The time from the reset to the end of `setup` goes to h2d_ms.
+template <class Setup>
+static int begin_ion(McsHandle* h, int32_t i_iter, int32_t i_ion, const McsSpecies* sp, long long n, long long first_global,
+                     Setup&& setup) {
+    CU(cudaSetDevice(h->device));
+    h->sp = *sp; h->i_iter = i_iter; h->i_ion = i_ion; h->reduced = false; h->ended = false; h->split_timed = false; h->last_steps_per_particle = 0;
+    h->n_use = n; h->first_global = first_global; h->n_saved_last = 0; h->n_saved_global_last = 0;
+    CU(cudaMemsetAsync(h->d_tally, 0, h->n_tally * 8, h->stream));
+    if (h->d_acc) CU(cudaMemsetAsync(h->d_acc, 0, h->n_tally * ACC_D * 8, h->stream));
+    CU(cudaMemsetAsync(h->d_u64, 0, (size_t)(h->ng + CNT_N) * 8, h->stream));
+    memset(h->h_counters, 0, sizeof h->h_counters);
+    CU(cudaEventRecord(h->ev2, h->stream));
+    const int rc = setup(h->pop[h->cur]);
+    if (rc) return rc;
+    CU(cudaEventRecord(h->ev3, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, h->ev2, h->ev3));
+    h->tm.h2d_ms += ms;
+    h->have_ion = true;
+    return MCS_OK;
+}
+
 extern "C" int mcs_begin_ion(McsHandle* h, int32_t i_iter, int32_t i_ion, const McsSpecies* sp, int64_t n, int64_t first_global,
                              const McsPopulation* pop) {
     if (!h || !sp || !pop) return fail(MCS_ERR_ARG, "null argument");
@@ -410,35 +419,18 @@ extern "C" int mcs_begin_ion(McsHandle* h, int32_t i_iter, int32_t i_ion, const 
     for (int64_t i = 0; i < n; i++)
         if (pop->grid[i] < 0 || pop->grid[i] > h->ng + 1) return fail(MCS_ERR_ARG, "grid index out of range");
     { int rcg = check_index_range(first_global, n); if (rcg) return rcg; }
-    CU(cudaSetDevice(h->device));
-    h->sp = *sp; h->i_iter = i_iter; h->i_ion = i_ion; h->reduced = false; h->ended = false; h->split_timed = false; h->last_steps_per_particle = 0;
-    h->n_use = n; h->first_global = first_global; h->n_saved_last = 0; h->n_saved_global_last = 0;
-    // clear_psd! (ion_init.jl:1-16) and every other per-ion sum
-    CU(cudaMemsetAsync(h->d_tally, 0, h->n_tally * 8, h->stream));
-    if (h->d_acc) CU(cudaMemsetAsync(h->d_acc, 0, h->n_tally * ACC_D * 8, h->stream));
-    CU(cudaMemsetAsync(h->d_u64, 0, (size_t)(h->ng + CNT_N) * 8, h->stream));
-    memset(h->h_counters, 0, sizeof h->h_counters);
-    CU(cudaEventRecord(h->ev2, h->stream));
-    PopPtrs& p = h->pop[h->cur];
-    size_t nb = (size_t)n * 8;
-#define UP(dst, src, bytes) do { if (src && n > 0) CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, h->stream)); } while (0)
-    UP(p.weight, pop->weight, nb); UP(p.ptot, pop->ptot_pf, nb); UP(p.pb, pop->pb_pf, nb); UP(p.x, pop->x_cm, nb);
-    UP(p.phi, pop->phi_rad, nb); UP(p.grid, pop->grid, nb); UP(p.xn_per, pop->xn_per, nb); UP(p.prp_x, pop->prp_x_cm, nb);
-    UP(p.acctime, pop->acctime_sec, nb); UP(p.tcut, pop->tcut, nb); UP(p.down, pop->downstream, (size_t)n); UP(p.inj, pop->inj, (size_t)n);
-#undef UP
-    if (n > 0) {
-        fill_defaults_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(
-            p, n, pop->downstream != nullptr, pop->inj != nullptr, pop->xn_per != nullptr, pop->prp_x_cm != nullptr,
-            pop->acctime_sec != nullptr, pop->tcut != nullptr, h->cfg.xn_per_fine, h->cfg.x_grid_stop);
+    return begin_ion(h, i_iter, i_ion, sp, n, first_global, [&](const PopPtrs& p) {
+        if (n == 0) return MCS_OK;
+        // every optional field gets its default first: the uploads of the fields the caller gives overwrite them
+        fill_defaults_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(p, n, h->cfg.xn_per_fine, h->cfg.x_grid_stop);
+        CU(cudaGetLastError());
         h->tm.other_launches++;
-    }
-    CU(cudaEventRecord(h->ev3, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, h->ev2, h->ev3));
-    h->tm.h2d_ms += ms;
-    h->have_ion = true;
-    return MCS_OK;
+#define X(T, name, pub) \
+        if (pop->pub) CU(cudaMemcpyAsync(p.name, pop->pub, (size_t)n * sizeof(T), cudaMemcpyHostToDevice, h->stream));
+        MCS_POP_FIELDS(X)
+#undef X
+        return MCS_OK;
+    });
 }
 
 extern "C" int mcs_begin_ion_generate(McsHandle* h, int32_t i_iter, int32_t i_ion, const McsSpecies* sp, int64_t first_global,
@@ -456,42 +448,30 @@ extern "C" int mcs_begin_ion_generate(McsHandle* h, int32_t i_iter, int32_t i_io
     if (inj->grid < 0 || inj->grid > h->ng + 1) return fail(MCS_ERR_ARG, "grid index out of range");
     { int rcg = check_index_range(first_global, n_local); if (rcg) return rcg; }
     if (n_total > 0x100000000ll) return fail(MCS_ERR_ARG, "global particle index exceeds 2^32 (RNG counter width)");
-    CU(cudaSetDevice(h->device));
-    h->sp = *sp; h->i_iter = i_iter; h->i_ion = i_ion; h->reduced = false; h->ended = false; h->split_timed = false; h->last_steps_per_particle = 0;
-    h->n_use = n_local; h->first_global = first_global; h->n_saved_last = 0; h->n_saved_global_last = 0;
-    CU(cudaMemsetAsync(h->d_tally, 0, h->n_tally * 8, h->stream));
-    if (h->d_acc) CU(cudaMemsetAsync(h->d_acc, 0, h->n_tally * ACC_D * 8, h->stream));
-    CU(cudaMemsetAsync(h->d_u64, 0, (size_t)(h->ng + CNT_N) * 8, h->stream));
-    memset(h->h_counters, 0, sizeof h->h_counters);
-    CU(cudaEventRecord(h->ev2, h->stream));
-    // bins: one packed upload [ptot | weight | lo | hi | gfac | start]
-    std::vector<double> pack((size_t)nb * 5 + (size_t)nb + 1, 0.0);
-    for (int b = 0; b < nb; b++) {
-        pack[b] = inj->bin_ptot[b]; pack[nb + b] = inj->bin_weight[b];
-        if (inj->mode != MCS_INJ_UPSTREAM) { pack[2 * nb + b] = inj->bin_lo[b]; pack[3 * nb + b] = inj->bin_hi[b]; pack[4 * nb + b] = inj->bin_gfac[b]; }
-    }
-    memcpy(&pack[(size_t)5 * nb], inj->bin_start, (size_t)(nb + 1) * 8);
-    cudaFree(h->d_inj); h->d_inj = nullptr;
-    CU(cudaMalloc(&h->d_inj, pack.size() * 8));
-    CU(cudaMemcpyAsync(h->d_inj, pack.data(), pack.size() * 8, cudaMemcpyHostToDevice, h->stream));
-    InjDev J;
-    J.ptot = h->d_inj; J.weight = h->d_inj + nb; J.lo = h->d_inj + 2 * nb; J.hi = h->d_inj + 3 * nb; J.gfac = h->d_inj + 4 * nb;
-    J.start = reinterpret_cast<const long long*>(h->d_inj + 5 * nb);
-    J.n_bins = nb; J.mode = inj->mode; J.perm_stride = inj->perm_stride; J.n_total = n_total; J.grid = inj->grid;
-    J.x_cm = inj->x_cm; J.u_stop = inj->u_stop; J.c = h->cfg.c_cms; J.xn_fine = h->cfg.xn_per_fine; J.x_grid_stop = h->cfg.x_grid_stop;
-    J.key0 = h->P.key0; J.key1 = h->P.key1; J.ctr2 = (uint32_t)i_ion << 16; J.ctr3 = (uint32_t)i_iter;
-    if (n_local > 0) {
-        generate_population_kernel<<<(unsigned)((n_local + 255) / 256), 256, 0, h->stream>>>(h->pop[h->cur], n_local, first_global, J);
-        CU(cudaGetLastError());
-        h->tm.other_launches++;
-    }
-    CU(cudaEventRecord(h->ev3, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, h->ev2, h->ev3));
-    h->tm.h2d_ms += ms;
-    h->have_ion = true;
-    return MCS_OK;
+    return begin_ion(h, i_iter, i_ion, sp, n_local, first_global, [&](const PopPtrs& p) {
+        // bins: one packed upload [ptot | weight | lo | hi | gfac | start]
+        std::vector<double> pack((size_t)nb * 5 + (size_t)nb + 1, 0.0);
+        for (int b = 0; b < nb; b++) {
+            pack[b] = inj->bin_ptot[b]; pack[nb + b] = inj->bin_weight[b];
+            if (inj->mode != MCS_INJ_UPSTREAM) { pack[2 * nb + b] = inj->bin_lo[b]; pack[3 * nb + b] = inj->bin_hi[b]; pack[4 * nb + b] = inj->bin_gfac[b]; }
+        }
+        memcpy(&pack[(size_t)5 * nb], inj->bin_start, (size_t)(nb + 1) * 8);
+        cudaFree(h->d_inj); h->d_inj = nullptr;
+        CU(cudaMalloc(&h->d_inj, pack.size() * 8));
+        CU(cudaMemcpyAsync(h->d_inj, pack.data(), pack.size() * 8, cudaMemcpyHostToDevice, h->stream));
+        InjDev J;
+        J.ptot = h->d_inj; J.weight = h->d_inj + nb; J.lo = h->d_inj + 2 * nb; J.hi = h->d_inj + 3 * nb; J.gfac = h->d_inj + 4 * nb;
+        J.start = reinterpret_cast<const long long*>(h->d_inj + 5 * nb);
+        J.n_bins = nb; J.mode = inj->mode; J.perm_stride = inj->perm_stride; J.n_total = n_total; J.grid = inj->grid;
+        J.x_cm = inj->x_cm; J.u_stop = inj->u_stop; J.c = h->cfg.c_cms; J.xn_fine = h->cfg.xn_per_fine; J.x_grid_stop = h->cfg.x_grid_stop;
+        J.key0 = h->P.key0; J.key1 = h->P.key1; J.ctr2 = (uint32_t)i_ion << 16; J.ctr3 = (uint32_t)i_iter;
+        if (n_local > 0) {
+            generate_population_kernel<<<(unsigned)((n_local + 255) / 256), 256, 0, h->stream>>>(p, n_local, first_global, J);
+            CU(cudaGetLastError());
+            h->tm.other_launches++;
+        }
+        return MCS_OK;
+    });
 }
 
 static int read_counters(McsHandle* h) {
@@ -631,6 +611,17 @@ static int compact_saved(McsHandle* h) {
     return MCS_OK;
 }
 
+// The end of an enqueued split: ev3 closes its timing bracket (opened with ev2) and the n_out children, the first of them
+// global index first_global, become the current population.
+static int finish_split(McsHandle* h, long long n_out, long long first_global, int64_t* n_new_local) {
+    CU(cudaEventRecord(h->ev3, h->stream));
+    h->split_timed = true;
+    int t = h->cur; h->cur = h->nxt; h->nxt = t;
+    h->n_use = n_out; h->first_global = first_global;
+    if (n_new_local) *n_new_local = n_out;
+    return MCS_OK;
+}
+
 // Single-rank split, enqueued only (the caller synchronises).  ev2/ev3 bracket it.
 static int split_local_async(McsHandle* h, int64_t i_mult, int64_t first_global_child, int64_t* n_new_local) {
     if (i_mult < 1) return fail(MCS_ERR_ARG, "i_mult < 1");
@@ -646,12 +637,7 @@ static int split_local_async(McsHandle* h, int64_t i_mult, int64_t first_global_
         CU(cudaGetLastError());
         h->tm.other_launches++;
     }
-    CU(cudaEventRecord(h->ev3, h->stream));
-    h->split_timed = true;
-    int t = h->cur; h->cur = h->nxt; h->nxt = t;
-    h->n_use = n_out; h->first_global = first_global_child;
-    if (n_new_local) *n_new_local = n_out;
-    return MCS_OK;
+    return finish_split(h, n_out, first_global_child, n_new_local);
 }
 
 static int sync_split_time(McsHandle* h) {
@@ -687,29 +673,27 @@ static int split_multi_async(McsHandle* h, const long long* ns_all, int64_t n_pt
     if (pe == SPLIT_PLAN_OVER_RANGE) return fail(MCS_ERR_ARG, "global particle index exceeds 2^32 (RNG counter width)");
     const GatherPrefix& pre = plan.pre;
     const long long i_mult = plan.i_mult, C = plan.C, c0 = plan.c0, n_out = plan.c1 - plan.c0, stride = plan.stride;
-    if ((size_t)stride * 82 * (size_t)h->nranks > h->xchg_bytes) return fail(MCS_ERR_STATE, "split exchange buffer too small");
+    const size_t block_bytes = (size_t)stride * POP_REC_BYTES;
+    if (block_bytes * (size_t)h->nranks > h->xchg_bytes) return fail(MCS_ERR_STATE, "split exchange buffer too small");
     CU(cudaEventRecord(h->ev2, h->stream));
     int rc = compact_saved(h);
     if (rc) return rc;
-    unsigned char* mine = h->d_xchg + (size_t)h->rank * (size_t)stride * 82;
+    unsigned char* mine = h->d_xchg + (size_t)h->rank * block_bytes;
     if (h->n_saved_last > 0) {
         pack_saved_kernel<<<(unsigned)((h->n_saved_last + 255) / 256), 256, 0, h->stream>>>(h->pop[1], h->d_saved_idx, h->n_saved_last,
                                                                                         mine, stride);
         CU(cudaGetLastError());
         h->tm.other_launches++;
     }
-    NC(g_nccl.AllGather(mine, h->d_xchg, (size_t)stride * 82, ncclUint8, h->comm, h->stream));
+    NC(g_nccl.AllGather(mine, h->d_xchg, block_bytes, ncclUint8, h->comm, h->stream));
     if (n_out > 0) {
         clone_gathered_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, h->stream>>>(h->d_xchg, stride, pre, h->pop[h->nxt], c0, n_out,
                                                                                    i_mult);
         CU(cudaGetLastError());
         h->tm.other_launches++;
     }
-    CU(cudaEventRecord(h->ev3, h->stream));
-    h->split_timed = true;
-    int t = h->cur; h->cur = h->nxt; h->nxt = t;
-    h->n_use = n_out; h->first_global = c0;
-    if (n_new_local) *n_new_local = n_out;
+    rc = finish_split(h, n_out, c0, n_new_local);
+    if (rc) return rc;
     if (n_new_global) *n_new_global = C;
     if (i_mult_out) *i_mult_out = i_mult;
     return MCS_OK;
@@ -956,22 +940,20 @@ extern "C" int mcs_get_population(McsHandle* h, int32_t which, int64_t n, McsPop
     if (!h || !o) return fail(MCS_ERR_ARG, "null argument");
     if (n < 0 || n > h->cfg.n_pts_max) return fail(MCS_ERR_ARG, "n out of range");
     CU(cudaSetDevice(h->device));
-    PopPtrs& p = which == 0 ? h->pop[h->cur] : h->pop[1];
-    size_t nb = (size_t)n * 8;
-#define DN(dst, src, bytes) do { if (dst && n > 0) CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, h->stream)); } while (0)
-    DN(o->weight, p.weight, nb); DN(o->ptot_pf, p.ptot, nb); DN(o->pb_pf, p.pb, nb); DN(o->x_cm, p.x, nb);
-    DN(o->xn_per, p.xn_per, nb); DN(o->prp_x_cm, p.prp_x, nb); DN(o->acctime_sec, p.acctime, nb); DN(o->phi_rad, p.phi, nb);
-    DN(o->grid, p.grid, nb); DN(o->tcut, p.tcut, nb); DN(o->downstream, p.down, (size_t)n); DN(o->inj, p.inj, (size_t)n);
-    DN(l_save, h->d_l_save, (size_t)n);
-#undef DN
+    const PopPtrs& p = which == 0 ? h->pop[h->cur] : h->pop[1];
+    if (n > 0) {
+#define X(T, name, pub) if (o->pub) CU(cudaMemcpyAsync(o->pub, p.name, (size_t)n * sizeof(T), cudaMemcpyDeviceToHost, h->stream));
+        MCS_POP_FIELDS(X)
+#undef X
+        if (l_save) CU(cudaMemcpyAsync(l_save, h->d_l_save, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+    }
     CU(cudaStreamSynchronize(h->stream));
     if (which == 1 && l_save) {  // reference zeroes the *_saved arrays (main_loops.jl:186-197): mask unsaved slots
         for (int64_t i = 0; i < n; i++) {
             if (l_save[i]) continue;
-            if (o->weight) o->weight[i] = 0; if (o->ptot_pf) o->ptot_pf[i] = 0; if (o->pb_pf) o->pb_pf[i] = 0;
-            if (o->x_cm) o->x_cm[i] = 0; if (o->xn_per) o->xn_per[i] = 0; if (o->prp_x_cm) o->prp_x_cm[i] = 0;
-            if (o->acctime_sec) o->acctime_sec[i] = 0; if (o->phi_rad) o->phi_rad[i] = 0; if (o->grid) o->grid[i] = 0;
-            if (o->tcut) o->tcut[i] = 0; if (o->downstream) o->downstream[i] = 0; if (o->inj) o->inj[i] = 0;
+#define X(T, name, pub) if (o->pub) o->pub[i] = 0;
+            MCS_POP_FIELDS(X)
+#undef X
         }
     }
     return MCS_OK;

@@ -87,11 +87,49 @@ enum : uint32_t {
     EV_REASON_SHIFT = 8, EV_XSPEC_SHIFT = 16,
 };
 
-struct PopPtrs {  // SoA particle record (main_loops.jl:212-226)
-    double *weight, *ptot, *pb, *x, *xn_per, *prp_x, *acctime, *phi;
-    long long *grid, *tcut;
-    uint8_t *down, *inj;
+// The particle record (main_loops.jl:212-226), one field per line in storage order: X(element type, PopPtrs member,
+// McsPopulation member).  The wider types come first, so in a block of pop_view's layout every field stays aligned.
+#define MCS_POP_FIELDS(X)              \
+    X(double, weight, weight)          \
+    X(double, ptot, ptot_pf)           \
+    X(double, pb, pb_pf)               \
+    X(double, x, x_cm)                 \
+    X(double, xn_per, xn_per)          \
+    X(double, prp_x, prp_x_cm)         \
+    X(double, acctime, acctime_sec)    \
+    X(double, phi, phi_rad)            \
+    X(long long, grid, grid)           \
+    X(long long, tcut, tcut)           \
+    X(uint8_t, down, downstream)       \
+    X(uint8_t, inj, inj)
+
+struct PopPtrs {  // SoA particle record: one array per field
+#define X(T, name, pub) T* name;
+    MCS_POP_FIELDS(X)
+#undef X
 };
+
+#define X(T, name, pub) +sizeof(T)
+constexpr size_t POP_REC_BYTES = 0 MCS_POP_FIELDS(X);  // bytes of one record
+#undef X
+#define X(T, name, pub) \
+    static_assert(sizeof *McsPopulation{}.pub == sizeof(T), "McsPopulation::" #pub " and PopPtrs::" #name " differ in size");
+MCS_POP_FIELDS(X)
+#undef X
+
+// n records rounded up to a multiple of 16: every f64 and i64 field of a block then starts a multiple of 128 bytes after it
+__host__ __device__ constexpr long long pop_cap(long long n) { return (n + 15) / 16 * 16; }
+
+// A population block: each field in turn holds `cap` records, in list order (POP_REC_BYTES * cap bytes).  The view
+// starts at record `first`.  The three populations of a handle and each rank's block of the split's exchange buffer
+// have this layout.
+__host__ __device__ inline PopPtrs pop_view(unsigned char* base, long long cap, long long first) {
+    PopPtrs p;
+#define X(T, name, pub) p.name = reinterpret_cast<T*>(base) + first; base += (size_t)cap * sizeof(T);
+    MCS_POP_FIELDS(X)
+#undef X
+    return p;
+}
 
 enum { SC_ESC_FLUX = 0, SC_PX_ESC_FEB, SC_EN_ESC_FEB, SC_SUMP, SC_SUMKE, SC_PX_ESC_UP, SC_EN_ESC_UP, SC_N = 8 };
 enum {
@@ -1951,39 +1989,36 @@ __global__ void pack_counts_kernel(const unsigned long long* __restrict__ counte
     out[1] = n_use; out[2] = err; out[3] = 0;
 }
 
+// record o of dst = record j of src, the weight divided by i_mult (cuts.jl:77; exact for i_mult = 1)
+__device__ __forceinline__ void copy_record(const PopPtrs& dst, long long o, const PopPtrs& src, long long j, long long i_mult) {
+#define X(T, name, pub) T name = src.name[j];
+    MCS_POP_FIELDS(X)
+#undef X
+    weight /= (double)i_mult;
+#define X(T, name, pub) dst.name[o] = name;
+    MCS_POP_FIELDS(X)
+#undef X
+}
+
+// child o of the split = copy of saved record saved_idx[o / i_mult]
 __global__ void clone_kernel(PopPtrs src, PopPtrs dst, const long long* __restrict__ saved_idx, long long n_out,
                              long long i_mult) {
     long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (o >= n_out) return;
-    long long j = saved_idx[o / i_mult];
-    dst.weight[o] = src.weight[j] / (double)i_mult;  // cuts.jl:77
-    dst.ptot[o] = src.ptot[j]; dst.pb[o] = src.pb[j]; dst.x[o] = src.x[j]; dst.grid[o] = src.grid[j];
-    dst.down[o] = src.down[j]; dst.inj[o] = src.inj[j]; dst.xn_per[o] = src.xn_per[j]; dst.prp_x[o] = src.prp_x[j];
-    dst.acctime[o] = src.acctime[j]; dst.phi[o] = src.phi[j]; dst.tcut[o] = src.tcut[j];
+    copy_record(dst, o, src, saved_idx[o / i_mult], i_mult);
 }
 
-// Multi-GPU split with rebalancing: every rank packs its saved records (SoA, padded to `stride` records) into its block of
-// a gather buffer; after ncclAllGather each rank clones an equal contiguous slice of the GLOBAL child index range.
-// Block layout (bytes): 8 f64 arrays | 2 i64 arrays | 2 u8 arrays, each `stride` long -> 82 * stride bytes.
+// Multi-GPU split with rebalancing: every rank packs its saved records into its block of an exchange buffer; block q is
+// pop_view(buf + q * stride * POP_REC_BYTES, stride, 0).  After ncclAllGather each rank clones an equal contiguous slice of
+// the GLOBAL child index range.
 struct GatherPrefix { long long start[65]; int nranks; };
 
-__device__ __forceinline__ unsigned char* gather_block(unsigned char* buf, int q, long long stride) {
-    return buf + (size_t)q * (size_t)stride * 82;
-}
-
+// record r of a rank's exchange block (`stride` records) = its saved record saved_idx[r], r < ns
 __global__ void pack_saved_kernel(PopPtrs src, const long long* __restrict__ saved_idx, long long ns, unsigned char* block,
                                   long long stride) {
     long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= ns) return;
-    const long long j = saved_idx[r];
-    double* f = reinterpret_cast<double*>(block);
-    f[r] = src.weight[j]; f[stride + r] = src.ptot[j]; f[2 * stride + r] = src.pb[j]; f[3 * stride + r] = src.x[j];
-    f[4 * stride + r] = src.xn_per[j]; f[5 * stride + r] = src.prp_x[j]; f[6 * stride + r] = src.acctime[j];
-    f[7 * stride + r] = src.phi[j];
-    long long* g = reinterpret_cast<long long*>(block + (size_t)stride * 64);
-    g[r] = src.grid[j]; g[stride + r] = src.tcut[j];
-    uint8_t* b = block + (size_t)stride * 80;
-    b[r] = src.down[j]; b[stride + r] = src.inj[j];
+    copy_record(pop_view(block, stride, 0), r, src, saved_idx[r], 1);
 }
 
 __global__ void clone_gathered_kernel(unsigned char* buf, long long stride, GatherPrefix pre, PopPtrs dst, long long c0,
@@ -1993,17 +2028,7 @@ __global__ void clone_gathered_kernel(unsigned char* buf, long long stride, Gath
     const long long sidx = (c0 + o) / i_mult;  // global rank of the saved parent (cuts.jl:69-91 order)
     int q = 0;
     while (q + 1 < pre.nranks && sidx >= pre.start[q + 1]) q++;
-    const long long r = sidx - pre.start[q];
-    const unsigned char* block = gather_block(buf, q, stride);
-    const double* f = reinterpret_cast<const double*>(block);
-    dst.weight[o] = f[r] / (double)i_mult;  // cuts.jl:77
-    dst.ptot[o] = f[stride + r]; dst.pb[o] = f[2 * stride + r]; dst.x[o] = f[3 * stride + r];
-    dst.xn_per[o] = f[4 * stride + r]; dst.prp_x[o] = f[5 * stride + r]; dst.acctime[o] = f[6 * stride + r];
-    dst.phi[o] = f[7 * stride + r];
-    const long long* g = reinterpret_cast<const long long*>(block + (size_t)stride * 64);
-    dst.grid[o] = g[r]; dst.tcut[o] = g[stride + r];
-    const uint8_t* b = block + (size_t)stride * 80;
-    dst.down[o] = b[r]; dst.inj[o] = b[stride + r];
+    copy_record(dst, o, pop_view(buf + (size_t)q * (size_t)stride * POP_REC_BYTES, stride, 0), sidx - pre.start[q], i_mult);
 }
 
 // Host plan of the rebalancing split for one rank, from every rank's saved count ns_all[0..nranks): the prefix of the
@@ -2041,7 +2066,7 @@ __host__ inline int split_plan(const long long* ns_all, int nranks, int rank, lo
     p->C = C;
     p->c0 = C * rank / nranks;
     p->c1 = C * (rank + 1) / nranks;
-    p->stride = (max_ns + 15) / 16 * 16;
+    p->stride = pop_cap(max_ns);
     return SPLIT_PLAN_OK;
 }
 
@@ -2105,16 +2130,14 @@ __global__ void sum_angle_kernel(const double* __restrict__ psd, int M2, int T2,
     dndp[idx] = s;
 }
 
-__global__ void fill_defaults_kernel(PopPtrs p, long long n, int has_down, int has_inj, int has_xn, int has_prp,
-                                     int has_acc, int has_tcut, double xn_fine, double x_grid_stop) {
+// the optional fields of a fresh record: upstream, not injected, the fine xn_per, prp_x at x_grid_stop, no age, tcut 1
+__device__ __forceinline__ void set_optional_defaults(const PopPtrs& p, long long i, double xn_fine, double x_grid_stop) {
+    p.down[i] = 0; p.inj[i] = 0; p.xn_per[i] = xn_fine; p.prp_x[i] = x_grid_stop; p.acctime[i] = 0.0; p.tcut[i] = 1;
+}
+
+__global__ void fill_defaults_kernel(PopPtrs p, long long n, double xn_fine, double x_grid_stop) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    if (!has_down) p.down[i] = 0;
-    if (!has_inj) p.inj[i] = 0;
-    if (!has_xn) p.xn_per[i] = xn_fine;
-    if (!has_prp) p.prp_x[i] = x_grid_stop;
-    if (!has_acc) p.acctime[i] = 0.0;
-    if (!has_tcut) p.tcut[i] = 1;
+    if (i < n) set_optional_defaults(p, i, xn_fine, x_grid_stop);
 }
 
 // init_pop in run-length form (include/mcs.h McsInjection; initializers.jl:977-1134, ion_init.jl:29-53).  HBM-bound: 82 B
@@ -2156,7 +2179,7 @@ __global__ void generate_population_kernel(PopPtrs p, long long n_local, long lo
     }
     p.weight[i] = J.weight[lo]; p.ptot[i] = ptot; p.pb[i] = pb; p.x[i] = J.x_cm; p.grid[i] = J.grid;
     p.phi[i] = __dmul_rn(TWO_PI, u2);
-    p.down[i] = 0; p.inj[i] = 0; p.xn_per[i] = J.xn_fine; p.prp_x[i] = J.x_grid_stop; p.acctime[i] = 0.0; p.tcut[i] = 1;
+    set_optional_defaults(p, i, J.xn_fine, J.x_grid_stop);
 }
 
 // sqrt_nr / div_nr against the IEEE operations on operands spread over the fast loop's ranges (mcs_math.cuh).

@@ -38,6 +38,18 @@ __global__ void k_asin_bf(const double* x, long n, double* y) {
     if (i < n) y[i] = asin_bf<NR>(x[i]);
 }
 
+// The split entry points take and return populations as three host arrays: the f64 fields, the i64 fields and the u8
+// fields, each field `cap` records long, in PopPtrs order.  They are the three consecutive byte ranges of one population
+// block of pop_view's layout, at[k]..at[k + 1], which start at its first field of each type.
+struct PopRanges {
+    unsigned char* at[4];
+    PopRanges(unsigned char* block, long long cap) {
+        const PopPtrs v = pop_view(block, cap, 0);
+        at[0] = reinterpret_cast<unsigned char*>(v.weight); at[1] = reinterpret_cast<unsigned char*>(v.grid); at[2] = v.down;
+        at[3] = block + (size_t)cap * POP_REC_BYTES;
+    }
+};
+
 // device buffers of one call, freed on every path out
 struct Bufs {
     void* p[16] = {};
@@ -60,6 +72,22 @@ struct Bufs {
     template <class T> void out(T* h, const T* d, size_t count) {
         if (err == cudaSuccess) err = cudaMemcpy(h, d, count * sizeof(T), cudaMemcpyDeviceToHost);
     }
+    // a population block of `cap` records from the three host arrays (PopRanges), and back
+    unsigned char* pop_in(const double* f64, const long long* i64, const uint8_t* u8, long long cap) {
+        unsigned char* d = alloc<unsigned char>((size_t)cap * POP_REC_BYTES);
+        if (!d) return nullptr;
+        const PopRanges r(d, cap);
+        const void* h[3] = {f64, i64, u8};
+        for (int k = 0; k < 3; k++)
+            if (err == cudaSuccess && r.at[k + 1] > r.at[k]) err = cudaMemcpy(r.at[k], h[k], r.at[k + 1] - r.at[k], cudaMemcpyHostToDevice);
+        return err == cudaSuccess ? d : nullptr;
+    }
+    void pop_out(double* f64, long long* i64, uint8_t* u8, unsigned char* d, long long cap) {
+        const PopRanges r(d, cap);
+        void* h[3] = {f64, i64, u8};
+        for (int k = 0; k < 3; k++)
+            if (err == cudaSuccess && r.at[k + 1] > r.at[k]) err = cudaMemcpy(h[k], r.at[k], r.at[k + 1] - r.at[k], cudaMemcpyDeviceToHost);
+    }
     int launched() {
         if (err == cudaSuccess) err = cudaGetLastError();
         if (err == cudaSuccess) err = cudaDeviceSynchronize();
@@ -67,19 +95,6 @@ struct Bufs {
     }
     ~Bufs() { for (int i = 0; i < n; i++) cudaFree(p[i]); }
 };
-
-// A population of `cap` records held field by field in three arrays, as the split entry points take it from the host:
-// f64 = 8 fields x cap in PopPtrs order (weight, ptot, pb, x, xn_per, prp_x, acctime, phi), i64 = grid, tcut,
-// u8 = down, inj.  The view starts at record `first`.
-PopPtrs pop_view(double* f64, long long* i64, uint8_t* u8, long long cap, long long first) {
-    PopPtrs p;
-    memset(&p, 0, sizeof p);
-    double** f[8] = {&p.weight, &p.ptot, &p.pb, &p.x, &p.xn_per, &p.prp_x, &p.acctime, &p.phi};
-    for (int k = 0; k < 8; k++) *f[k] = f64 + k * cap + first;
-    p.grid = i64 + first; p.tcut = i64 + cap + first;
-    p.down = u8 + first; p.inj = u8 + cap + first;
-    return p;
-}
 
 }  // namespace
 
@@ -175,7 +190,7 @@ int du_asin_bf(const double* x, long n, int nr, double* y) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// The split of new_pcut.  Populations cross in the field-major layout of pop_view.
+// The split of new_pcut.  Populations are held in blocks of pop_view's layout, as in the library.
 
 // enqueue_compaction on l_save[0..n): saved_idx gets all n entries (zero past *total)
 int du_compact(const uint8_t* l_save, long n, long long* saved_idx, long long* total) {
@@ -200,18 +215,14 @@ int du_split_local(const double* f64, const long long* i64, const uint8_t* u8, c
                    long cap, double* out_f64, long long* out_i64, uint8_t* out_u8, long long* total) {
     if (i_mult < 1) return cudaErrorInvalidValue;
     Bufs b;
-    double* d_f = b.in(f64, 8 * (size_t)n);
-    long long* d_i = b.in(i64, 2 * (size_t)n);
-    uint8_t* d_u = b.in(u8, 2 * (size_t)n);
+    unsigned char* d_pop = b.pop_in(f64, i64, u8, n);
     const uint8_t* d_l = b.in(l_save, n);
     const long long nb = compaction_blocks(n);
     int* d_cnt = b.alloc<int>(nb);
     long long* d_off = b.alloc<long long>(nb);
     long long* d_total = b.alloc<long long>(1);
     long long* d_idx = b.alloc<long long>(n);
-    double* o_f = b.alloc<double>(8 * (size_t)cap);
-    long long* o_i = b.alloc<long long>(2 * (size_t)cap);
-    uint8_t* o_u = b.alloc<uint8_t>(2 * (size_t)cap);
+    unsigned char* o_pop = b.alloc<unsigned char>((size_t)cap * POP_REC_BYTES);
     if (b.err) return b.err;
     if (n > 0) enqueue_compaction(d_l, n, d_cnt, d_off, d_total, d_idx, 0);
     b.launched();
@@ -220,9 +231,9 @@ int du_split_local(const double* f64, const long long* i64, const uint8_t* u8, c
     const long long n_out = *total * i_mult;
     if (n_out > cap) return cudaErrorInvalidValue;
     if (n_out > 0)
-        clone_kernel<<<blocks(n_out), TPB>>>(pop_view(d_f, d_i, d_u, n, 0), pop_view(o_f, o_i, o_u, cap, 0), d_idx, n_out, i_mult);
+        clone_kernel<<<blocks(n_out), TPB>>>(pop_view(d_pop, n, 0), pop_view(o_pop, cap, 0), d_idx, n_out, i_mult);
     b.launched();
-    b.out(out_f64, o_f, 8 * (size_t)cap); b.out(out_i64, o_i, 2 * (size_t)cap); b.out(out_u8, o_u, 2 * (size_t)cap);
+    b.pop_out(out_f64, out_i64, out_u8, o_pop, cap);
     return b.err;
 }
 
@@ -243,9 +254,7 @@ int du_split_ranks(int nranks, const long long* n_per_rank, const uint8_t* l_sav
     }
     const long long N = first[nranks];
     Bufs b;
-    double* d_f = b.in(f64, 8 * (size_t)N);
-    long long* d_i = b.in(i64, 2 * (size_t)N);
-    uint8_t* d_u = b.in(u8, 2 * (size_t)N);
+    unsigned char* d_pop = b.pop_in(f64, i64, u8, N);
     const uint8_t* d_l = b.in(l_save, N);
     int* d_cnt = b.alloc<int>(nb_max);
     long long* d_off = b.alloc<long long>(nb_max);
@@ -263,23 +272,21 @@ int du_split_ranks(int nranks, const long long* n_per_rank, const uint8_t* l_sav
         if (split_plan(ns_all, nranks, r, target, n_pts_max, &plan[r]) != SPLIT_PLAN_OK) return cudaErrorInvalidValue;
     const long long stride = plan[0].stride;
     if (plan[0].C > cap) return cudaErrorInvalidValue;
-    unsigned char* d_x = b.alloc<unsigned char>((size_t)nranks * (size_t)stride * 82);
-    double* o_f = b.alloc<double>(8 * (size_t)cap);
-    long long* o_i = b.alloc<long long>(2 * (size_t)cap);
-    uint8_t* o_u = b.alloc<uint8_t>(2 * (size_t)cap);
+    unsigned char* d_x = b.alloc<unsigned char>((size_t)nranks * (size_t)stride * POP_REC_BYTES);
+    unsigned char* o_pop = b.alloc<unsigned char>((size_t)cap * POP_REC_BYTES);
     if (b.err) return b.err;
     for (int q = 0; q < nranks; q++)
         if (ns_all[q] > 0)
-            pack_saved_kernel<<<blocks(ns_all[q]), TPB>>>(pop_view(d_f, d_i, d_u, N, first[q]), d_idx + first[q], ns_all[q],
-                                                          d_x + (size_t)q * (size_t)stride * 82, stride);
+            pack_saved_kernel<<<blocks(ns_all[q]), TPB>>>(pop_view(d_pop, N, first[q]), d_idx + first[q], ns_all[q],
+                                                          d_x + (size_t)q * (size_t)stride * POP_REC_BYTES, stride);
     for (int r = 0; r < nranks; r++) {
         n_out[r] = plan[r].c1 - plan[r].c0;
         if (n_out[r] > 0)
-            clone_gathered_kernel<<<blocks(n_out[r]), TPB>>>(d_x, stride, plan[r].pre, pop_view(o_f, o_i, o_u, cap, plan[r].c0),
-                                                             plan[r].c0, n_out[r], plan[r].i_mult);
+            clone_gathered_kernel<<<blocks(n_out[r]), TPB>>>(d_x, stride, plan[r].pre, pop_view(o_pop, cap, plan[r].c0), plan[r].c0,
+                                                             n_out[r], plan[r].i_mult);
     }
     b.launched();
-    b.out(out_f64, o_f, 8 * (size_t)cap); b.out(out_i64, o_i, 2 * (size_t)cap); b.out(out_u8, o_u, 2 * (size_t)cap);
+    b.pop_out(out_f64, out_i64, out_u8, o_pop, cap);
     *i_mult = plan[0].i_mult;
     return b.err;
 }
